@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the KLHR hot path (BASELINE.json metric: chain-draws/sec, ESS/sec, % roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     torchrun --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Headline workload (BASELINE.json configs[1]): stan/ill-normal, D = 100 diagonal Gaussian, 65 536 chains per GPU,
@@ -19,8 +19,14 @@ The JSON line also carries
   e2e       the metric through the public sampler API from pinned HOST buffers; e2e_sample: MCMCBase.sample's own
             contract (every draw returned, mcmc.py:31-37) streamed to pinned host memory;
   configs   BASELINE.json configs[2..4] (funnel + sinh-arcsinh family, dense corr-normal D = 256, arK T = 10 000)
-            measured the same way, each with its roofline and its adaptation phase (c5 is the config whose
-            closure all-reduce runs over every rank of --gpus N).
+            measured the same way, --steps timed steps each, with its roofline and its adaptation phase (c5 is the
+            config whose closure all-reduce runs over every rank of --gpus N).
+
+`--dump-outputs DIR` writes, on rank 0, what the last timed step of each workload left to its caller -- the chain states
+(`<tag>_theta.npy`, chains x D, the sampler's dtype) and the per-chain accept counts (`<tag>_accept_count.npy`,
+float64) -- for comparing two builds output for output: every input derives from a fixed seed, so the same arguments
+give the same inputs.  At most 64 MB in all: a workload whose arrays exceed its share keeps a fixed, seeded sample of
+chains (the same chains in both of its files).
 
 `--impl reference` times the reference's own CPU implementation of the same step (the SciPy-BFGS single-chain port in
 oracle/ref_port.py, one process per chain on all host cores, like reference run_experiments:27) -- /root/reference
@@ -64,7 +70,12 @@ def parse_args():
                     help="cudaProfilerStart/Stop around the first timed launch of that config (ncu --profile-from-start off)")
     ap.add_argument("--ref-draws-per-step", type=int, default=400)
     ap.add_argument("--ref-procs", type=int, default=0, help="0 = all host cores")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of each workload to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 # =============================================================================== CPU reference arm
@@ -238,6 +249,23 @@ def ark_series(T=10_000, K=5):
     return y[500:]
 
 
+DUMP_MB = {"c2": 55, "c3": 2, "c3_dims11": 2, "c4": 2, "c5": 2}    # shares of the <= 64 MB --dump-outputs writes
+
+
+def last_step_outputs(tag, sampler):
+    """`<tag>_theta` and `<tag>_accept_count` of `sampler` as host arrays (the sampler's dtype / float64); a sampler
+    whose two arrays exceed the workload's share of DUMP_MB keeps the same fixed, seeded sample of chains in both."""
+    import numpy as np
+    import torch
+    theta, acc = sampler._theta, sampler._accept_count
+    rows = DUMP_MB[tag] * 10 ** 6 // (theta.shape[1] * theta.element_size() + 8)
+    if theta.shape[0] > rows:
+        idx = np.sort(np.random.default_rng(SEED).choice(theta.shape[0], rows, replace=False))
+        idx = torch.as_tensor(idx, device=theta.device)
+        theta, acc = theta[idx], acc[idx]
+    return {f"{tag}_theta": theta.cpu().numpy(), f"{tag}_accept_count": acc.double().cpu().numpy()}
+
+
 def run_b200(args):
     import numpy as np
     import torch
@@ -264,6 +292,10 @@ def run_b200(args):
     B, D, S, K, W = args.chains, args.dim, args.draws_per_step, args.steps, args.warmup
     rb = 8 if dtype == torch.float64 else 4
     launches = [0]                                   # klhr_run launches inside timed regions (gpu_launches)
+    dumps = None
+    if args.dump_outputs and rank == 0:
+        dumps = {}
+        Path(args.dump_outputs).mkdir(parents=True, exist_ok=True)
 
     trace_on = bool(os.environ.get("KLHR_BENCH_TRACE"))
     t_start = time.time()
@@ -385,6 +417,8 @@ def run_b200(args):
         lambda: kb.KLHR(model, seed=SEED, chains=B, warmup=args.adapt_warmup, windowsize=50, windowscale=2,
                         dtype=dtype, device=dev), args.adapt_warmup)     # windows close at 50,150,350,1000 (+ all-reduce)
     total_ms, (wall0, wall1) = timed_steps(sampler, S, K, W, True, "c2")
+    if dumps is not None:
+        dumps.update(last_step_outputs("c2", sampler))          # before the e2e arm moves the chains on
     value = world * B * S * K / (total_ms * 1e-3)
     info = kb.launch_info(model, sampler._fit, dtype=dtype, free_running=True, accumulate=False, device=dev)
 
@@ -502,20 +536,20 @@ def run_b200(args):
     cfg_lines = {}
     # =============================================================== configs[2..4]
     if not args.no_configs:
-        Kc = max(3, min(K, 5))
-
         def run_config(tag, workload, make_sampler, draws, hbm_bytes_per_draw, peak_tflops, peak_name, kernel, note, extra=None,
                        alg_flops=None):
             smp, a_s, a_cold = adapt_phase(make_sampler, 1000)
             a_draws = world * smp.chains * 1000
-            t_ms, (c0_, c1_) = timed_steps(smp, draws, Kc, max(W, 3), False, tag)
-            val = world * smp.chains * draws * Kc / (t_ms * 1e-3)
+            t_ms, (c0_, c1_) = timed_steps(smp, draws, K, max(W, 3), False, tag)
+            if dumps is not None:
+                dumps.update(last_step_outputs(tag, smp))
+            val = world * smp.chains * draws * K / (t_ms * 1e-3)
             trace(f"{tag}: timed steps done")
             ev0 = int(smp._evals_total.item())
             smp.run(draws)
             evals = (int(smp._evals_total.item()) - ev0) / (smp.chains * draws)
             trace(f"{tag}: evaluation count done")
-            out = {"workload": workload, "value": val, "unit": UNIT, "ms_per_step": t_ms / Kc, "steps": Kc,
+            out = {"workload": workload, "value": val, "unit": UNIT, "ms_per_step": t_ms / K, "steps": K,
                    "draws_per_step": draws, "chains_per_gpu": smp.chains, "acceptance": smp.acceptance_probability,
                    "line_evaluations_per_draw": evals,
                    "adapt": {"draws": 1000, "closures": smp._windowedadaptation.closures, "phase_s": a_s, "cold_phase_s": a_cold,
@@ -611,6 +645,8 @@ def run_b200(args):
         if world == 1 and not args.no_cpu_baseline:
             cb, _ = cpu_baseline(D, 2000, args.ref_procs, args.adapt_warmup)
             line["cpu_baseline"] = cb
+        for name, a in (dumps or {}).items():
+            np.save(Path(args.dump_outputs) / f"{name}.npy", a)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -35,6 +35,35 @@ def test_gpu_arm_refuses_to_run_without_a_device():
     assert out.returncode != 0 and "no CPU fallback" in (out.stderr + out.stdout)
 
 
+def test_dump_outputs_fit_their_share_and_keep_a_fixed_sample_of_chains():
+    """`--dump-outputs`: every workload's arrays fit its share of DUMP_MB (64 MB in all, .npy headers included); a larger
+    sampler keeps a seeded sample of chains, the same in theta and the accept counts and the same run after run."""
+    import types
+    import numpy as np
+    import torch
+    sys.path.insert(0, str(ROOT))
+    import bench
+    assert sum(bench.DUMP_MB.values()) < 64
+    B, D = 4096, 256
+    smp = types.SimpleNamespace(_theta=torch.arange(B * D, dtype=torch.float64).reshape(B, D),
+                                _accept_count=torch.arange(B))
+    out = bench.last_step_outputs("c4", smp)
+    th, acc = out["c4_theta"], out["c4_accept_count"]
+    assert th.dtype == acc.dtype == np.float64 and th.nbytes + acc.nbytes <= bench.DUMP_MB["c4"] * 10 ** 6
+    assert 0 < len(acc) < B and th.shape == (len(acc), D) and len(np.unique(acc)) == len(acc)
+    assert np.array_equal(th[:, 0] / D, acc)                           # the same chains in both files
+    again = bench.last_step_outputs("c4", smp)
+    assert all(np.array_equal(out[k], again[k]) for k in out)
+    small = types.SimpleNamespace(_theta=torch.ones(64, 100, dtype=torch.float32), _accept_count=torch.zeros(64, dtype=torch.int64))
+    out = bench.last_step_outputs("c2", small)                          # under its share: every chain
+    assert out["c2_theta"].dtype == np.float32 and out["c2_theta"].shape == (64, 100) and out["c2_accept_count"].shape == (64,)
+    # the headline workload at its default size is written whole
+    assert 65_536 * (100 * 8 + 8) <= bench.DUMP_MB["c2"] * 10 ** 6
+    ref = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--dump-outputs", "x"],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert ref.returncode != 0 and "--dump-outputs needs --impl b200" in ref.stderr
+
+
 def test_normals_accounting_follows_the_lane_kernels_element_map():
     """`roofline.normals.generated_per_chain_draw` against a walk of the lane kernel's sweep (csrc/klhr_lane.cuh): trip t
     covers the coordinate quads at e = 32 (t // 2) + 4 (t % 2) + 8 r, r = 0..3, and draws 16 normals whatever part of it
