@@ -189,8 +189,8 @@ int klhr_run(const klhr_model_t* model, const klhr_fit_t* fit, const klhr_direct
 
 /* Random-walk Metropolis (reference mh.py:7-37, the comparison sampler of experiment_accuracy.py:69) on
  * the same engine: n_steps draws theta' = theta + stepsize N(0, I) per chain with the chain's Philox
- * stream.  accum: accept_count, draws/thin, chain_s1/chain_s2 are honoured; trace: rho receives xi,
- * plus r, accept, u. */
+ * stream.  accum: accept_count, draws/thin, chain_s1/chain_s2 (+shift) are honoured; pooled_s1/pooled_s2
+ * are refused; trace: rho receives xi, plus r, accept, u. */
 int klhr_mh_run(const klhr_model_t* model, int dtype, void* theta_dev, double stepsize, int64_t n_chains,
                 int64_t chain_offset, int64_t draw_offset, int32_t n_steps, uint64_t seed,
                 const klhr_accum_t* accum, const klhr_trace_t* trace, void* stream);

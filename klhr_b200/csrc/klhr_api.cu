@@ -373,13 +373,18 @@ int klhr_mh_run(const klhr_model_t* model, int dtype, void* theta_dev, double st
     if (dtype != KLHR_F64 && dtype != KLHR_F32) return fail(-9, "dtype must be KLHR_F64 or KLHR_F32");
     if (n_chains < 0 || n_steps < 0 || chain_offset < 0 || draw_offset < 0) return fail(-10, "negative count or offset");
     if (!(stepsize > 0)) return fail(-14, "stepsize must be positive");
+    a.acc.thin = 1;
+    if (accum) {
+        a.acc = *accum;
+        if (a.acc.thin < 1) a.acc.thin = 1;
+        if (a.acc.pooled_s1 || a.acc.pooled_s2) return fail(-12, "klhr_mh_run: pooled in-kernel moments are not supported");
+        if (a.acc.chain_s2 && !a.acc.chain_s1) return fail(-12, "chain_s2 needs chain_s1");
+    }
+    if (trace) a.tr = *trace;
     if (n_chains == 0 || n_steps == 0) return 0;
     if (!theta_dev) return fail(-1, "theta must not be NULL");
     a.theta = theta_dev; a.B = n_chains; a.stepsize = stepsize;
     a.chain_offset = chain_offset; a.draw_offset = draw_offset; a.n_steps = n_steps; a.seed = seed;
-    a.acc.thin = 1;
-    if (accum) { a.acc = *accum; if (a.acc.thin < 1) a.acc.thin = 1; }
-    if (trace) a.tr = *trace;
     cudaStream_t st = (cudaStream_t)stream;
     int e = -2;
     switch (a.mp.id) {

@@ -141,9 +141,10 @@ __device__ __forceinline__ void dk_tri_product(const XT* __restrict__ rows, int 
 }
 
 // sum over the kDkLpc consecutive lanes that share a chain
-__device__ __forceinline__ double dk_grp_sum(double v) {
+// gmask: the lanes of the chain's group only -- the groups of a ragged last CTA that hold no chain skip the call
+__device__ __forceinline__ double dk_grp_sum(double v, unsigned gmask) {
 #pragma unroll
-    for (int off = 1; off < kDkLpc; off <<= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+    for (int off = 1; off < kDkLpc; off <<= 1) v += __shfl_xor_sync(gmask, v, off);
     return v;
 }
 
@@ -253,7 +254,10 @@ __global__ void __launch_bounds__(kDkThreads, 32 / kDkChains) dense_kernel(const
                         s_lu[o] = lg;                          // log of the accept uniform, off the critical path of the fit
                     }
                 }
-                const R u_col = __shfl_sync(0xffffffffu, sv0, 0, LPC);
+                // group mask, not the full warp: in a ragged last CTA a warp can hold valid and invalid chains, and
+                // only the valid groups get here
+                const unsigned gmask = (LPC == 32 ? 0xffffffffu : ((1u << LPC) - 1u)) << (LPC * (lane / LPC));
+                const R u_col = __shfl_sync(gmask, sv0, 0, LPC);
                 int jcol = 0;
                 if (n_cols > 1)                                // searchsorted(cdf, u, 'right'), klhr.py:147
                     while (jcol < n_cols - 1 && (float)u_col >= s_cdf[jcol]) ++jcol;
@@ -279,7 +283,7 @@ __global__ void __launch_bounds__(kDkThreads, 32 / kDkChains) dense_kernel(const
                         }
                     }
                 }
-                ss = dk_grp_sum(ss);
+                ss = dk_grp_sum(ss, gmask);
                 if (j == 0) s_inv[o] = R(1) / r_sqrt(ss);      // rho = x / ||x + tol||  (klhr.py:153)
             }
         }

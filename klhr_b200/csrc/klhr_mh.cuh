@@ -96,11 +96,14 @@ __global__ void __launch_bounds__(kThreadsMax) mh_kernel(const __grid_constant__
                 for (int i = lane; i < D; i += kOct) g[i] = th[i];
             }
         }
-        if (a.acc.chain_s1)
+        if (a.acc.chain_s1) {
+            const R* sh = reinterpret_cast<const R*>(a.acc.shift);
             for (int i = lane; i < D; i += kOct) {
-                a.acc.chain_s1[c * D + i] += (double)th[i];
-                if (a.acc.chain_s2) a.acc.chain_s2[c * D + i] += (double)th[i] * (double)th[i];
+                const double d = (double)th[i] - (sh ? (double)sh[i] : 0.0);
+                a.acc.chain_s1[c * D + i] += d;
+                if (a.acc.chain_s2) a.acc.chain_s2[c * D + i] += d * d;
             }
+        }
     }
     for (int i = lane; i < D; i += kOct) g_theta[c * D + i] = th[i];
     if (lane == 0 && a.acc.accept_count) a.acc.accept_count[c] += n_acc;

@@ -26,11 +26,12 @@ class MH(MCMCBase):
         self._chain_offset = int(chain_offset)
         self._accept_count = torch.zeros(self.chains, dtype=torch.int64, device=self.device)
 
-    def _advance(self, n, draws=None, thin=1, chain_s1=None, chain_s2=None, trace=None):
+    def _advance(self, n, draws=None, thin=1, chain_s1=None, chain_s2=None, trace=None, shift=None, thin_offset=0):
         lib = _lib.load()
         md = self.model.descriptor(self.dtype, self.device)
         ad = _lib.AccumDesc(accept_count=_ptr(self._accept_count), draws=_ptr(draws), thin=int(thin),
-                            chain_s1=_ptr(chain_s1), chain_s2=_ptr(chain_s2), thin_offset=0)
+                            chain_s1=_ptr(chain_s1), chain_s2=_ptr(chain_s2), shift=_ptr(shift),
+                            thin_offset=int(thin_offset))
         trd = trace.descriptor() if trace is not None else None
         with torch.cuda.device(self.device):
             st = torch.cuda.current_stream(self.device).cuda_stream

@@ -34,6 +34,16 @@ def fit_pair(family, dtype=torch.float64, **kw):
     return k, o
 
 
+# replay tapes of the unmodified reference (tests/golden) by line family
+GAUSS_TAPES = ["normal_d2_klhr", "normal_d2_klhr_method2", "illnormal_d100_klhr",
+               "illnormal_d100_klhr_tight", "corrnormal_n50_klhr", "ar1_n100_klhr",
+               "funnel_d2_klhr", "funnel_d2_klhr_tight", "funnel_d11_klhr_tight",
+               "ark_t200_klhr_tight", "rosenbrock_d4_klhr_tight", "earnings_klhr_tight",
+               "illnormal_d20_klhr_scaledir"]
+SINH_TAPES = ["funnel_d2_sinh", "funnel_d2_sinh_tight", "ark_t200_sinh", "rosenbrock_d4_sinh", "earnings_sinh",
+              "funnel_d2_sinh_scaledir_method1",
+              "funnel_d2_subsinh_tight", "rosenbrock_d4_subsinh"]     # subsinh: SUBKLHRSINH, d = 1 (sub_klhr_sinh.py)
+
 DIAG_MODELS = ("normal", "ill-normal")     # targets the tile kernel covers (csrc/klhr_tile.cuh)
 
 

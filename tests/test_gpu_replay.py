@@ -7,18 +7,9 @@ import pytest
 import torch
 
 from conftest import load_tape
-from gpu_util import replay_both, rel_errors
+from gpu_util import GAUSS_TAPES, SINH_TAPES, replay_both, rel_errors
 
 pytestmark = pytest.mark.gpu
-
-GAUSS_TAPES = ["normal_d2_klhr", "normal_d2_klhr_method2", "illnormal_d100_klhr",
-               "illnormal_d100_klhr_tight", "corrnormal_n50_klhr", "ar1_n100_klhr",
-               "funnel_d2_klhr", "funnel_d2_klhr_tight", "funnel_d11_klhr_tight",
-               "ark_t200_klhr_tight", "rosenbrock_d4_klhr_tight", "earnings_klhr_tight",
-               "illnormal_d20_klhr_scaledir"]
-SINH_TAPES = ["funnel_d2_sinh", "funnel_d2_sinh_tight", "ark_t200_sinh", "rosenbrock_d4_sinh", "earnings_sinh",
-              "funnel_d2_sinh_scaledir_method1",
-              "funnel_d2_subsinh_tight", "rosenbrock_d4_subsinh"]     # subsinh: SUBKLHRSINH, d = 1 (sub_klhr_sinh.py)
 
 
 def _run(name, dtype, force_octet=False):
