@@ -209,8 +209,18 @@ constexpr uint32_t kSlotAccept = 2;    // w0,w1: 53-bit accept uniform
 constexpr uint32_t kSlotInit4 = 3;     // w0..w3: two Box-Muller pairs -> init4[2], init4[3] (sinh)
 constexpr uint32_t kSlotDir = 8;       // direction element i: slot kSlotDir + (i % 8) + 8 ((i % 128) / 32) + 32 (i / 128), word (i % 32) / 8
 
-// uniform in (0,1) from 32 bits: (x + 0.5) / 2^32
+// uniform from the top 24 bits: (x >> 8 + 0.5) / 2^24, rounded to fp32.  The range is [2^-25, 1], not (0, 1): from
+// 1/2 up the lattice points fall halfway between fp32 neighbours and round to even, the top one (x >= 0xFFFFFF00,
+// probability 2^-24) to exactly 1.0.  Where this uniform is used that is harmless: a Box-Muller radius of 0 (one zero
+// normal), the last direction column, a rejected draw (log u = 0), a slice candidate at the bracket end, a binomial
+// trial P(u < u0) off u0 by at most 2^-24.  Exponentials must not be formed from it: see exp1_32.
 __device__ __forceinline__ float u01_32(uint32_t x) { return fmaf((float)(x >> 8), 1.0f / 16777216.0f, 0.5f / 16777216.0f); }
+// -log u of the same lattice point u = (x >> 8 + 0.5) / 2^24, an Exp(1) variate: -log u below 1/2, where u is exact
+// in fp32, and -log1p(-(1 - u)) from 1/2 up, where 1 - u is the lattice point of ~x, exact as well.  So it is never 0
+// and keeps fp32 relative accuracy (logf, log1pf: 1 ulp) down to its smallest value 2^-25.
+__device__ __forceinline__ float exp1_32(uint32_t x) {
+    return x < 0x80000000u ? -logf(u01_32(x)) : -log1pf(-u01_32(~x));
+}
 // uniform in (0,1) from 53 of 64 bits
 __device__ __forceinline__ double u01_53(uint32_t hi, uint32_t lo) {
     const uint64_t v = (((uint64_t)hi << 32) | lo) >> 11;

@@ -499,26 +499,24 @@ __device__ inline void overrelax_sample(OrCtx<R>& oc, R u0) {
     const int K = oc.K;
     uint32_t w[4];
     int have = 0, q = 0;
-    auto next_u = [&]() -> float {
+    auto next_word = [&]() -> uint32_t {
         if (have == 0) {
             Philox::block(oc.c0, oc.c1, oc.d0, 0x80000000u + (uint32_t)q, oc.k0, oc.k1d, w);
             ++q;
             have = 4;
         }
-        const float x = u01_32(w[4 - have]);
-        --have;
-        return x;
+        return w[4 - have--];
     };
     int r = 0;
-    for (int k = 0; k < K; ++k) r += ((R)next_u() < u0) ? 1 : 0;
+    for (int k = 0; k < K; ++k) r += ((R)u01_32(next_word()) < u0) ? 1 : 0;
     int na = 0, nb = 0;
     if (r > K - r) { na = K - r + 1; nb = 2 * r - K; }
     else if (r < K - r) { na = r + 1; nb = K - 2 * r; }
     R v = 1;
     if (na > 0) {                // Beta(a, b), integer a, b: Ga / (Ga + Gb) with Gamma(n) = -sum log U
         float ga = 0, gb = 0;
-        for (int i = 0; i < na; ++i) ga -= __logf(next_u());
-        for (int i = 0; i < nb; ++i) gb -= __logf(next_u());
+        for (int i = 0; i < na; ++i) ga += exp1_32(next_word());
+        for (int i = 0; i < nb; ++i) gb += exp1_32(next_word());
         v = (R)(ga / (ga + gb));
     }
     oc.r = r;

@@ -74,6 +74,30 @@ def replay_both(model_name, data, family, theta, rho, z_init, z_prop, u, init4=N
     return gpu, ref
 
 
+def _pad(D, rb):
+    """pad_dim of csrc/klhr_step.cuh."""
+    mod = 16 if rb == 8 else 32
+    p = -(-D // mod) * mod + 8
+    return p - mod if p - mod >= D else p
+
+
+def assert_kernel(model, kfit, dtype, want, accumulate=False, free_running=True):
+    """The launch plan of ``want`` (csrc: launch_lane / launch_tile_typed / chain_smem_bytes / plan_step /
+    densek_smem_bytes / launch_densews_nt) is the one the dispatcher picks for this model, fit and dtype."""
+    info = kb.launch_info(model, kfit, dtype=dtype, free_running=free_running, accumulate=accumulate, device=device())
+    D, rb, t, sm = model.dim(), 8 if dtype == torch.float64 else 4, info["threads"], info["smem"]
+    ok = {
+        "lane": t == 64,
+        "tile": t == 32 and sm == ((D + 1) & ~1) * rb + 32 * _pad(D, 4) * 4 + D * 4,
+        "chain_serial": D <= 16 and t == 32 and sm == (64 * (D | 1) + D) * rb,
+        "chain_octet": D > 16 and t == 32 and sm == (36 * _pad(D, rb) + D) * rb,
+        "octet": t % 32 == 0 and sm == ((4 if accumulate else 2) * (t // 8) * _pad(D, rb) + 2 * D) * rb,
+        "dense_ws": t == 512,
+        "dense": t == 256 and sm == 2 * 32 * (D + 4) * 8 + 8 * 4 * (D // 64) * 64 * 8 + (8 * 32 * 2 + 6 * 32) * 8 + D * 4,
+    }[want]
+    assert ok, (want, info)
+
+
 def rel_errors(gpu, ref, family):
     """Dimensionless errors: m and zp in units of the fitted scale s, log-parameters absolute."""
     s = np.exp(np.clip(ref["eta"][:, 1], -300, 300))

@@ -12,7 +12,7 @@ import pytest
 import torch
 
 import klhr_b200 as kb
-from gpu_util import GAUSS_TAPES, SINH_TAPES, device, fit_pair, rel_errors, replay_both, up
+from gpu_util import GAUSS_TAPES, SINH_TAPES, assert_kernel, device, fit_pair, rel_errors, replay_both, up
 from oracle import batched, stan_models
 from oracle.ref_port import gauss_hermite_probabilists
 
@@ -63,30 +63,6 @@ def test_mh_run_refuses_pooled_moments_and_a_lone_chain_s2():
 
 
 # ---------------------------------------------------------------------------------------------------- helpers
-def _pad(D, rb):
-    """pad_dim of csrc/klhr_step.cuh."""
-    mod = 16 if rb == 8 else 32
-    p = -(-D // mod) * mod + 8
-    return p - mod if p - mod >= D else p
-
-
-def _assert_kernel(model, kfit, dtype, want, accumulate=False, free_running=True):
-    """The launch plan of ``want`` (csrc: launch_lane / launch_tile_typed / chain_smem_bytes / plan_step /
-    densek_smem_bytes / launch_densews_nt) is the one the dispatcher picks for this model, fit and dtype."""
-    info = kb.launch_info(model, kfit, dtype=dtype, free_running=free_running, accumulate=accumulate, device=device())
-    D, rb, t, sm = model.dim(), 8 if dtype == F64 else 4, info["threads"], info["smem"]
-    ok = {
-        "lane": t == 64,
-        "tile": t == 32 and sm == ((D + 1) & ~1) * rb + 32 * _pad(D, 4) * 4 + D * 4,
-        "chain_serial": D <= 16 and t == 32 and sm == (64 * (D | 1) + D) * rb,
-        "chain_octet": D > 16 and t == 32 and sm == (36 * _pad(D, rb) + D) * rb,
-        "octet": t % 32 == 0 and sm == ((4 if accumulate else 2) * (t // 8) * _pad(D, rb) + 2 * D) * rb,
-        "dense_ws": t == 512,
-        "dense": t == 256 and sm == 2 * 32 * (D + 4) * 8 + 8 * 4 * (D // 64) * 64 * 8 + (8 * 32 * 2 + 6 * 32) * 8 + D * 4,
-    }[want]
-    assert ok, (want, info)
-
-
 def _direction(D, dtype=F64):
     """An adapted-looking direction law: two stored mean columns, one zero column, non-unit sd."""
     cols = np.zeros((2, D))
@@ -178,7 +154,7 @@ def test_dense_kernel_replay_evaluation_and_accept_counts(N, rho, B):
     the oracle's on every chain, ragged last CTA included."""
     data = {"N": N, "rho": rho}
     model = kb.BSModel(stan_file="stan/corr-normal.stan", data=data, device=device())
-    _assert_kernel(model, _kfit("gauss", F64)[0], F64, "dense", free_running=False)
+    assert_kernel(model, _kfit("gauss", F64)[0], F64, "dense", free_running=False)
     rng = np.random.default_rng(N + B)
     theta = rng.normal(size=(B, N)) * 0.7
     r = rng.normal(size=(B, N))
@@ -231,8 +207,8 @@ def test_free_running_evaluation_and_accept_counts(case):
     model = kb.BSModel(stan_file=f"stan/{name}.stan", data=data, device=device())
     om = stan_models.make_model(name, data)
     kfit, ofit = _kfit(family, dtype, force, or_K)
-    _assert_kernel(model, kfit, dtype, kernel)
-    _assert_kernel(model, kfit, dtype, kernel_rows, free_running=kernel_rows != "dense")
+    assert_kernel(model, kfit, dtype, kernel)
+    assert_kernel(model, kfit, dtype, kernel_rows, free_running=kernel_rows != "dense")
     D, S = model.dim(), 5
     rng = np.random.default_rng(B + D)
     theta0 = rng.normal(size=(B, D)) * 0.3
@@ -331,7 +307,7 @@ def test_step_kernel_moment_sums_shift_and_skip_accum_last(name, data, dtype, B)
     each launch; shift=None gives raw sums."""
     model = kb.BSModel(stan_file=f"stan/{name}.stan", data=data, device=device())
     kfit, _ = _kfit("gauss", dtype)
-    _assert_kernel(model, kfit, dtype, "octet", accumulate=True)
+    assert_kernel(model, kfit, dtype, "octet", accumulate=True)
     D, S, cut = model.dim(), 60, 25
     rng = np.random.default_rng(D)
     theta0 = _f32(rng.normal(size=(B, D)) * 0.3)
@@ -442,7 +418,7 @@ def test_thinned_rows_across_a_launch_cut(case):
     cid, name, data, family, force, dtype, kernel, bitwise = case
     model = kb.BSModel(stan_file=f"stan/{name}.stan", data=data, device=device())
     kfit, _ = _kfit(family, dtype, force)
-    _assert_kernel(model, kfit, dtype, kernel, free_running=kernel != "dense")
+    assert_kernel(model, kfit, dtype, kernel, free_running=kernel != "dense")
     D, B, M = model.dim(), 333, 4
     rng = np.random.default_rng(7)
     theta0 = rng.normal(size=(B, D)) * 0.3
@@ -528,8 +504,8 @@ def test_fp32_free_running_step_equals_oracle_on_emitted_variates(name, data, fo
     om = stan_models.make_model(name, data)
     kfit, ofit = _kfit("gauss", F32, "octet" if force_octet else None)
     D, B, S = model.dim(), 500, 3
-    _assert_kernel(model, kfit, F32, "octet" if force_octet else
-                   "tile" if name in ("normal", "ill-normal") else "chain_serial" if D <= 16 else "chain_octet")
+    assert_kernel(model, kfit, F32, "octet" if force_octet else
+                  "tile" if name in ("normal", "ill-normal") else "chain_serial" if D <= 16 else "chain_octet")
     theta0 = _f32(np.random.default_rng(D).normal(size=(B, D)) * 0.3)
     th, acc, ev, t, _ = _traced_run(model, kfit, theta0, F32, (1, 2), 17, _direction(D, F32))
     assert ev == int(t["evals"].astype(np.int64).sum()) and np.array_equal(acc, t["accept"].astype(np.int64).sum(0))
