@@ -42,7 +42,11 @@ enum {
     KLHR_MODEL_ARK = 5,         /* stan/arK.stan          i0 = K, i1 = T-K, data0 = [G|c|yy]      */
     KLHR_MODEL_ROSENBROCK = 6,  /* stan/rosenbrock.stan   i0 = D; dim = 2 D                       */
     KLHR_MODEL_EARNINGS = 7,    /* stan/earnings.stan     data0 = [N, Se, Sh, See, Seh, Shh]; dim = 4 */
-    KLHR_MODEL_COUNT = 8
+    KLHR_MODEL_EIGHT_SCHOOLS_NC = 8, /* posteriordb eight_schools_noncentered  i0 = J, data0 = [y_1..J | w_1..J],
+                                        w = 1/sigma^2; dim = J + 2, order [theta_trans, mu, log tau] */
+    KLHR_MODEL_EIGHT_SCHOOLS_C = 9,  /* posteriordb eight_schools_centered     i0 = J, data0 = [y_1..J | w_1..J],
+                                        w = 1/sigma^2; dim = J + 2, order [mu, log tau, theta]       */
+    KLHR_MODEL_COUNT = 10
 };
 
 /* Target density descriptor (replaces a bridgestan.StanModel handle, bsmodel.py:10-13). */

@@ -35,6 +35,28 @@ def _dtype_code(dtype):
         raise TypeError(f"klhr_b200 computes in float64 or float32, not {dtype}") from None
 
 
+_EIGHT_SCHOOLS = ("eight_schools_noncentered", "eight_schools_centered")
+
+
+def _eight_schools_data(d):
+    """(J, y, sigma) of the eight-schools data block, validated: J >= 1, y and sigma of length J, sigma > 0 and finite."""
+    try:
+        J = int(d["J"])
+        y = np.asarray(d["y"], dtype=np.float64)
+        sigma = np.asarray(d["sigma"], dtype=np.float64)
+    except (KeyError, TypeError) as e:
+        raise ValueError(f"eight schools: data needs J, y[J] and sigma[J] ({e})") from None
+    if J < 1 or J != d["J"]:
+        raise ValueError(f"eight schools: J must be an integer >= 1, got {d['J']!r}")
+    if y.shape != (J,) or sigma.shape != (J,):
+        raise ValueError(f"eight schools: y and sigma must have length J = {J}, got {y.shape} and {sigma.shape}")
+    if not np.all(np.isfinite(y)):
+        raise ValueError("eight schools: y must be finite")
+    if not np.all(np.isfinite(sigma) & (sigma > 0)):
+        raise ValueError("eight schools: sigma must be positive and finite")
+    return J, y, sigma
+
+
 class BSModel:
     def __init__(self, stan_file="", data_file="", stepsize=1.0, warn=False, data=None, device=None):
         self._stan_file = stan_file
@@ -105,6 +127,9 @@ class BSModel:
             if e.shape != (int(d["N"]),) or ht.shape != e.shape:
                 raise ValueError("earnings: earn and height must have length N")
             h.update(dim=4, data0=np.array([float(len(e)), e.sum(), ht.sum(), e @ e, e @ ht, ht @ ht]))
+        elif n in _EIGHT_SCHOOLS:                    # posteriordb eight_schools_{noncentered,centered}
+            J, y, sigma = _eight_schools_data(d)
+            h.update(dim=J + 2, i0=J, data0=np.concatenate([y, 1.0 / (sigma * sigma)]))
         return h
 
     def dim(self):
@@ -179,6 +204,9 @@ class BSModel:
             out[..., -1] = torch.exp(out[..., -1]) if torch.is_tensor(out) else np.exp(out[..., -1])
         if self.name == "earnings":                  # sigma, s > 0, stan/earnings.stan:9-10
             out[..., 2:] = torch.exp(out[..., 2:]) if torch.is_tensor(out) else np.exp(out[..., 2:])
+        if self.name in _EIGHT_SCHOOLS:              # tau = exp(u)
+            k = self._tau_index()
+            out[..., k] = torch.exp(out[..., k]) if torch.is_tensor(out) else np.exp(out[..., k])
         return out
 
     def unconstrain(self, theta):
@@ -187,7 +215,14 @@ class BSModel:
             out[..., -1] = torch.log(out[..., -1]) if torch.is_tensor(out) else np.log(out[..., -1])
         if self.name == "earnings":
             out[..., 2:] = torch.log(out[..., 2:]) if torch.is_tensor(out) else np.log(out[..., 2:])
+        if self.name in _EIGHT_SCHOOLS:
+            k = self._tau_index()
+            out[..., k] = torch.log(out[..., k]) if torch.is_tensor(out) else np.log(out[..., k])
         return out
+
+    def _tau_index(self):
+        """Position of tau (unconstrained: log tau) in the parameter vector of the eight-schools programs."""
+        return self._host["i0"] + 1 if self.name == "eight_schools_noncentered" else 1
 
     def parameter_names(self):
         h = self._host
@@ -199,6 +234,10 @@ class BSModel:
             return ["beta.1", "beta.2", "sigma", "s"]
         if self.name == "rosenbrock":
             return [f"v.{i + 1}" for i in range(h["i0"])] + [f"theta.{i + 1}" for i in range(h["i0"])]
+        if self.name == "eight_schools_noncentered":
+            return [f"theta_trans.{j + 1}" for j in range(h["i0"])] + ["mu", "tau"]
+        if self.name == "eight_schools_centered":
+            return ["mu", "tau"] + [f"theta.{j + 1}" for j in range(h["i0"])]
         return [f"y.{i + 1}" for i in range(h["dim"])]
 
     def Hamiltonian(self, theta, rho):               # bsmodel.py:45-46

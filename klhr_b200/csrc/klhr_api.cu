@@ -60,6 +60,11 @@ static int check_model(const klhr_model_t* m, ModelParams& mp) {
         case KLHR_MODEL_EARNINGS:
             if (!m->data0 || m->dim != 4) return fail(-5, "earnings: need data0 = [N,Se,Sh,See,Seh,Shh], dim = 4");
             break;
+        case KLHR_MODEL_EIGHT_SCHOOLS_NC:
+        case KLHR_MODEL_EIGHT_SCHOOLS_C:
+            if (!m->data0 || m->i0 < 1 || m->dim != m->i0 + 2)
+                return fail(-5, "eight schools: need data0 = [y|w], i0 = J >= 1, dim = J + 2");
+            break;
         default: break;
     }
     return 0;
@@ -127,6 +132,8 @@ static int dispatch_chain(const StepArgs& a, int dtype, int family, bool replay,
         case KLHR_MODEL_ARK: return launch_chain_ark(a, dtype, family, replay, st, info);
         case KLHR_MODEL_ROSENBROCK: return launch_chain_rosenbrock(a, dtype, family, replay, st, info);
         case KLHR_MODEL_EARNINGS: return launch_chain_earnings(a, dtype, family, replay, st, info);
+        case KLHR_MODEL_EIGHT_SCHOOLS_NC: return launch_chain_eight_schools_nc(a, dtype, family, replay, st, info);
+        case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_chain_eight_schools_c(a, dtype, family, replay, st, info);
     }
     return fail(-2, "unknown model id");
 }
@@ -146,6 +153,8 @@ static int dispatch_step(const StepArgs& a, int dtype, int family, bool replay, 
         case KLHR_MODEL_ARK: return launch_step_ark(a, dtype, family, replay, accum, st, info);
         case KLHR_MODEL_ROSENBROCK: return launch_step_rosenbrock(a, dtype, family, replay, accum, st, info);
         case KLHR_MODEL_EARNINGS: return launch_step_earnings(a, dtype, family, replay, accum, st, info);
+        case KLHR_MODEL_EIGHT_SCHOOLS_NC: return launch_step_eight_schools_nc(a, dtype, family, replay, accum, st, info);
+        case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_step_eight_schools_c(a, dtype, family, replay, accum, st, info);
     }
     return fail(-2, "unknown model id");
 }
@@ -288,6 +297,8 @@ int klhr_model_eval(const klhr_model_t* model, int dtype, const void* theta_dev,
         case KLHR_MODEL_ARK: e = launch_eval_ark(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
         case KLHR_MODEL_ROSENBROCK: e = launch_eval_rosenbrock(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
         case KLHR_MODEL_EARNINGS: e = launch_eval_earnings(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
+        case KLHR_MODEL_EIGHT_SCHOOLS_NC: e = launch_eval_eight_schools_nc(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
+        case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_eval_eight_schools_c(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
     }
     return cuda_fail(e, "klhr_model_eval");
 }
@@ -396,6 +407,8 @@ int klhr_mh_run(const klhr_model_t* model, int dtype, void* theta_dev, double st
         case KLHR_MODEL_ARK: e = launch_mh_ark(a, dtype, st); break;
         case KLHR_MODEL_ROSENBROCK: e = launch_mh_rosenbrock(a, dtype, st); break;
         case KLHR_MODEL_EARNINGS: e = launch_mh_earnings(a, dtype, st); break;
+        case KLHR_MODEL_EIGHT_SCHOOLS_NC: e = launch_mh_eight_schools_nc(a, dtype, st); break;
+        case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_mh_eight_schools_c(a, dtype, st); break;
     }
     return cuda_fail(e, "klhr_mh_run");
 }
@@ -419,6 +432,8 @@ static int dispatch_slice(const SliceArgs& a, int dtype, bool replay, cudaStream
         case KLHR_MODEL_ARK: return launch_slice_ark(a, dtype, replay, st);
         case KLHR_MODEL_ROSENBROCK: return launch_slice_rosenbrock(a, dtype, replay, st);
         case KLHR_MODEL_EARNINGS: return launch_slice_earnings(a, dtype, replay, st);
+        case KLHR_MODEL_EIGHT_SCHOOLS_NC: return launch_slice_eight_schools_nc(a, dtype, replay, st);
+        case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_slice_eight_schools_c(a, dtype, replay, st);
     }
     return -2;
 }
@@ -503,6 +518,8 @@ int klhr_kl_eval(const klhr_model_t* model, const klhr_fit_t* fit, int dtype, co
         case KLHR_MODEL_ARK: e = launch_kl_ark(a, dtype, fit->family, st); break;
         case KLHR_MODEL_ROSENBROCK: e = launch_kl_rosenbrock(a, dtype, fit->family, st); break;
         case KLHR_MODEL_EARNINGS: e = launch_kl_earnings(a, dtype, fit->family, st); break;
+        case KLHR_MODEL_EIGHT_SCHOOLS_NC: e = launch_kl_eight_schools_nc(a, dtype, fit->family, st); break;
+        case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_kl_eight_schools_c(a, dtype, fit->family, st); break;
     }
     return cuda_fail(e, "klhr_kl_eval");
 }

@@ -378,5 +378,7 @@ KLHR_DECLARE_MODEL_CHAIN(ar1)
 KLHR_DECLARE_MODEL_CHAIN(ark)
 KLHR_DECLARE_MODEL_CHAIN(rosenbrock)
 KLHR_DECLARE_MODEL_CHAIN(earnings)
+KLHR_DECLARE_MODEL_CHAIN(eight_schools_nc)
+KLHR_DECLARE_MODEL_CHAIN(eight_schools_c)
 
 }  // namespace klhr

@@ -144,5 +144,7 @@ KLHR_DECLARE_MODEL_MH(ar1)
 KLHR_DECLARE_MODEL_MH(ark)
 KLHR_DECLARE_MODEL_MH(rosenbrock)
 KLHR_DECLARE_MODEL_MH(earnings)
+KLHR_DECLARE_MODEL_MH(eight_schools_nc)
+KLHR_DECLARE_MODEL_MH(eight_schools_c)
 
 }  // namespace klhr

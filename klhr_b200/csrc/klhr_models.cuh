@@ -510,4 +510,205 @@ struct Earnings {
     }
 };
 
+// ------------------------------------------------------------------ eight schools (hierarchical normal)
+// Data (both parametrisations): i0 = J, data0 = [y_1..J | w_1..J] in R, w_j = 1 / sigma_j^2.  u = log tau.
+//
+// The half-Cauchy prior on tau, on the unconstrained scale, is -log1p(tau^2 / 25) = -softplus(z), z = 2u - log 25.
+// log1p(exp(2u) / 25) overflows from u ~ 355 (fp64) or ~ 45 (fp32), long before the line searches of the fit stop
+// visiting such u; the stable form max(z, 0) + log1p(e^-|z|) is finite wherever z is, and its derivatives come from
+// the logistic function sigma(z) = d softplus / dz.  e^-|z| is formed from the model's own exponential (e^{2u} / 25
+// or its reciprocal), so an evaluation costs one exponential and one log1p.
+template <typename R>
+struct Softplus { R sp, sg, sg1; };          // softplus(z), sigma(z), sigma(z) (1 - sigma(z))
+
+template <typename R>
+__device__ __forceinline__ Softplus<R> softplus_q(R z, R q /* e^-|z| */) {
+    Softplus<R> s;
+    const R inv = R(1) / (R(1) + q);
+    s.sp = r_max(z, R(0)) + r_log1p(q);
+    s.sg = z >= R(0) ? inv : q * inv;
+    s.sg1 = q * inv * inv;
+    return s;
+}
+
+// e^-|z| for z = 2u - log 25 from e2 = e^{2u}: 25 / e2 above u = log 5, e2 / 25 below
+template <typename R>
+__device__ __forceinline__ R cauchy_q_from_e2(R z, R e2) { return z >= R(0) ? R(25) / e2 : e2 * R(1.0 / 25.0); }
+
+constexpr double kLog25 = 3.2188758248682006;
+
+// ---- posteriordb eight_schools_noncentered   params [theta_trans_1..J, mu, u = log tau]
+//   data { int<lower=0> J; real y[J]; real<lower=0> sigma[J]; }
+//   parameters { vector[J] theta_trans; real mu; real<lower=0> tau; }
+//   transformed parameters { vector[J] theta = theta_trans * tau + mu; }
+//   model { theta_trans ~ normal(0, 1); y ~ normal(theta, sigma); mu ~ normal(0, 5); tau ~ cauchy(0, 5); }
+// lp = -1/2 sum tt^2 - 1/2 sum w (y - mu - e^u tt)^2 - mu^2 / 50 - softplus(2u - log 25) + u.
+// Line tt = a + t r, mu = m0 + t rm, u = u0 + t ru, c = y - m0, d = c - t rm: with W(f) = sum_j w_j f_j the
+// likelihood sum is P(t) - 2 e^u Q(t) + e^{2u} S(t), P = sum w d^2, Q = sum w d tt, S = sum w tt^2, all quadratics
+// in t.  Everything but e^u Q - e^{2u} S / 2 - softplus is a quadratic in t, kept as its change b1 t + b2 t^2 from
+// t = 0 (the constants W(c^2), sum a^2 cancel, so 11 of the 13 sums are needed).
+template <typename R>
+struct EightSchoolsNC {
+    using Self = EightSchoolsNC<R>;
+    static constexpr bool kDenseCta = false;
+    struct Coef { R b1, b2, q0, q1, q2, s0, s1, s2, u0, ru, f0; };
+    __device__ static __forceinline__ R y_(int j, const ModelParams& mp) { return __ldg(reinterpret_cast<const R*>(mp.p0) + j); }
+    __device__ static __forceinline__ R w_(int j, const ModelParams& mp) {
+        return __ldg(reinterpret_cast<const R*>(mp.p0) + mp.i0 + j);
+    }
+    // e^u Q - e^{2u} S / 2 - softplus(z) and its first two t-derivatives
+    __device__ static __forceinline__ Jet<R> nonpoly(const Coef& c, R y) {
+        const R u = c.u0 + y * c.ru;
+        const R E = r_exp(u), e2 = E * E;
+        const R z = R(2) * u - R(kLog25);
+        const Softplus<R> s = softplus_q(z, cauchy_q_from_e2(z, e2));
+        const R Q = c.q0 + y * (c.q1 + y * c.q2), Q1 = c.q1 + R(2) * y * c.q2, Q2 = R(2) * c.q2;
+        const R S = c.s0 + y * (c.s1 + y * c.s2), S1 = c.s1 + R(2) * y * c.s2, S2 = R(2) * c.s2;
+        Jet<R> j;
+        j.l = E * Q - R(0.5) * e2 * S - s.sp;
+        j.l1 = E * (c.ru * Q + Q1) - R(0.5) * e2 * (R(2) * c.ru * S + S1) - R(2) * c.ru * s.sg;
+        j.l2 = E * (c.ru * c.ru * Q + R(2) * c.ru * Q1 + Q2) - R(0.5) * e2 * (R(4) * c.ru * c.ru * S + R(4) * c.ru * S1 + S2)
+               - R(4) * c.ru * c.ru * s.sg1;
+        return j;
+    }
+    template <int GS = kOct>
+    __device__ static Coef setup(const R* th, const R* rh, int lane, unsigned m, const ModelParams& mp) {
+        const int J = mp.i0;
+        const R m0 = th[J], rm = rh[J];
+        R W1 = 0, Wc = 0, Wa = 0, Wr = 0, Wca = 0, Wcr = 0, Wa2 = 0, War = 0, Wr2 = 0, ar = 0, r2 = 0;
+        for (int j = lane; j < J; j += GS) {
+            const R w = w_(j, mp), c = y_(j, mp) - m0, a = th[j], r = rh[j];
+            W1 += w; Wc += w * c; Wa += w * a; Wr += w * r;
+            Wca += w * c * a; Wcr += w * c * r;
+            Wa2 += w * a * a; War += w * a * r; Wr2 += w * r * r;
+            ar += a * r; r2 += r * r;
+        }
+        W1 = grp_sum<GS>(W1, m); Wc = grp_sum<GS>(Wc, m); Wa = grp_sum<GS>(Wa, m); Wr = grp_sum<GS>(Wr, m);
+        Wca = grp_sum<GS>(Wca, m); Wcr = grp_sum<GS>(Wcr, m);
+        Wa2 = grp_sum<GS>(Wa2, m); War = grp_sum<GS>(War, m); Wr2 = grp_sum<GS>(Wr2, m);
+        ar = grp_sum<GS>(ar, m); r2 = grp_sum<GS>(r2, m);
+        Coef c;
+        c.u0 = th[J + 1];
+        c.ru = rh[J + 1];
+        // -1/2 sum tt^2 - 1/2 P - mu^2 / 50 + u, less its value at t = 0
+        c.b1 = -ar + rm * Wc - m0 * rm * R(1.0 / 25.0) + c.ru;
+        c.b2 = -R(0.5) * r2 - R(0.5) * rm * rm * W1 - rm * rm * R(1.0 / 50.0);
+        c.q0 = Wca; c.q1 = Wcr - rm * Wa; c.q2 = -rm * Wr;
+        c.s0 = Wa2; c.s1 = R(2) * War; c.s2 = Wr2;
+        c.f0 = 0;
+        c.f0 = nonpoly(c, R(0)).l;
+        return c;
+    }
+    __device__ static __forceinline__ Jet<R> eval(const Coef& c, R y) {
+        const Jet<R> f = nonpoly(c, y);
+        return jet_guard<R>(y * (c.b1 + y * c.b2) + f.l - c.f0, c.b1 + R(2) * y * c.b2 + f.l1, R(2) * c.b2 + f.l2);
+    }
+    KLHR_DEFAULT_EVAL_CLIP
+    template <int G = kOct>
+    __device__ static R lp_grad(const R* th, R* g, int lane, unsigned m, const ModelParams& mp) {
+        const int J = mp.i0;
+        const R mu = th[J], u = th[J + 1];
+        const R E = r_exp(u);
+        R acc = 0, swr = 0, swrt = 0;
+        for (int j = lane; j < J; j += G) {
+            const R tt = th[j], w = w_(j, mp);
+            const R res = y_(j, mp) - mu - E * tt;
+            acc -= R(0.5) * (tt * tt + w * res * res);
+            swr += w * res;
+            swrt += w * res * tt;
+            if (g) g[j] = -tt + E * w * res;
+        }
+        acc = grp_sum<G>(acc, m); swr = grp_sum<G>(swr, m); swrt = grp_sum<G>(swrt, m);
+        const R z = R(2) * u - R(kLog25);
+        const Softplus<R> s = softplus_q(z, cauchy_q_from_e2(z, E * E));
+        if (g && lane == 0) {
+            g[J] = swr - mu * R(1.0 / 25.0);
+            g[J + 1] = E * swrt - R(2) * s.sg + R(1);
+        }
+        return acc - mu * mu * R(1.0 / 50.0) - s.sp + u;
+    }
+};
+
+// ---- posteriordb eight_schools_centered   params [mu, u = log tau, theta_1..J]
+//   data { int<lower=0> J; real y[J]; real<lower=0> sigma[J]; }
+//   parameters { real mu; real<lower=0> tau; real theta[J]; }
+//   model { mu ~ normal(0, 5); tau ~ cauchy(0, 5); theta ~ normal(mu, tau); y ~ normal(theta, sigma); }
+// lp = -mu^2 / 50 - softplus(2u - log 25) + (1 - J) u - 1/2 e^{-2u} sum (theta - mu)^2 - 1/2 sum w (y - theta)^2.
+// Line theta = a + t r, mu = m0 + t rm, u = u0 + t ru: sum (theta - mu)^2 = A0 + 2 A1 t + A2 t^2 and
+// sum w (y - theta)^2 = B0 - 2 B1 t + B2 t^2 (B0 cancels in l(t) - l(0)).
+template <typename R>
+struct EightSchoolsC {
+    using Self = EightSchoolsC<R>;
+    static constexpr bool kDenseCta = false;
+    struct Coef { R b1, b2, A0, A1, A2, u0, ru, f0; };
+    __device__ static __forceinline__ R y_(int j, const ModelParams& mp) { return __ldg(reinterpret_cast<const R*>(mp.p0) + j); }
+    __device__ static __forceinline__ R w_(int j, const ModelParams& mp) {
+        return __ldg(reinterpret_cast<const R*>(mp.p0) + mp.i0 + j);
+    }
+    // -1/2 e^{-2u} A(t) - softplus(z) and its first two t-derivatives
+    __device__ static __forceinline__ Jet<R> nonpoly(const Coef& c, R y) {
+        const R u = c.u0 + y * c.ru;
+        const R em2 = r_exp(-R(2) * u);
+        const R z = R(2) * u - R(kLog25);
+        const Softplus<R> s = softplus_q(z, z >= R(0) ? R(25) * em2 : R(1) / (R(25) * em2));
+        const R A = c.A0 + y * (R(2) * c.A1 + y * c.A2), A1 = R(2) * (c.A1 + y * c.A2), A2 = R(2) * c.A2;
+        Jet<R> j;
+        j.l = -R(0.5) * em2 * A - s.sp;
+        j.l1 = -R(0.5) * em2 * (A1 - R(2) * c.ru * A) - R(2) * c.ru * s.sg;
+        j.l2 = -R(0.5) * em2 * (R(4) * c.ru * c.ru * A - R(4) * c.ru * A1 + A2) - R(4) * c.ru * c.ru * s.sg1;
+        return j;
+    }
+    template <int GS = kOct>
+    __device__ static Coef setup(const R* th, const R* rh, int lane, unsigned m, const ModelParams& mp) {
+        const int J = mp.i0;
+        const R m0 = th[0], rm = rh[0];
+        R A0 = 0, A1 = 0, A2 = 0, B1 = 0, B2 = 0;
+        for (int j = lane; j < J; j += GS) {
+            const R w = w_(j, mp), a = th[2 + j], r = rh[2 + j];
+            const R dm = a - m0, dr = r - rm, e = y_(j, mp) - a;
+            A0 += dm * dm; A1 += dm * dr; A2 += dr * dr;
+            B1 += w * e * r; B2 += w * r * r;
+        }
+        Coef c;
+        c.A0 = grp_sum<GS>(A0, m); c.A1 = grp_sum<GS>(A1, m); c.A2 = grp_sum<GS>(A2, m);
+        B1 = grp_sum<GS>(B1, m); B2 = grp_sum<GS>(B2, m);
+        c.u0 = th[1];
+        c.ru = rh[1];
+        // -mu^2 / 50 + (1 - J) u - 1/2 sum w (y - theta)^2, less its value at t = 0
+        c.b1 = -m0 * rm * R(1.0 / 25.0) + R(1 - J) * c.ru + B1;
+        c.b2 = -rm * rm * R(1.0 / 50.0) - R(0.5) * B2;
+        c.f0 = 0;
+        c.f0 = nonpoly(c, R(0)).l;
+        return c;
+    }
+    __device__ static __forceinline__ Jet<R> eval(const Coef& c, R y) {
+        const Jet<R> f = nonpoly(c, y);
+        return jet_guard<R>(y * (c.b1 + y * c.b2) + f.l - c.f0, c.b1 + R(2) * y * c.b2 + f.l1, R(2) * c.b2 + f.l2);
+    }
+    KLHR_DEFAULT_EVAL_CLIP
+    template <int G = kOct>
+    __device__ static R lp_grad(const R* th, R* g, int lane, unsigned m, const ModelParams& mp) {
+        const int J = mp.i0;
+        const R mu = th[0], u = th[1];
+        const R em2 = r_exp(-R(2) * u);
+        R sd = 0, sd2 = 0, lik = 0;
+        for (int j = lane; j < J; j += G) {
+            const R tj = th[2 + j], w = w_(j, mp);
+            const R d = tj - mu, e = y_(j, mp) - tj;
+            sd += d;
+            sd2 += d * d;
+            lik += w * e * e;
+            if (g) g[2 + j] = -em2 * d + w * e;
+        }
+        sd = grp_sum<G>(sd, m); sd2 = grp_sum<G>(sd2, m); lik = grp_sum<G>(lik, m);
+        const R z = R(2) * u - R(kLog25);
+        const Softplus<R> s = softplus_q(z, z >= R(0) ? R(25) * em2 : R(1) / (R(25) * em2));
+        if (g && lane == 0) {
+            g[0] = -mu * R(1.0 / 25.0) + em2 * sd;
+            g[1] = -R(2) * s.sg + R(1 - J) + em2 * sd2;
+        }
+        return -mu * mu * R(1.0 / 50.0) - s.sp + R(1 - J) * u - R(0.5) * em2 * sd2 - R(0.5) * lik;
+    }
+};
+
 }  // namespace klhr

@@ -233,5 +233,7 @@ KLHR_DECLARE_MODEL_SLICE(ar1)
 KLHR_DECLARE_MODEL_SLICE(ark)
 KLHR_DECLARE_MODEL_SLICE(rosenbrock)
 KLHR_DECLARE_MODEL_SLICE(earnings)
+KLHR_DECLARE_MODEL_SLICE(eight_schools_nc)
+KLHR_DECLARE_MODEL_SLICE(eight_schools_c)
 
 }  // namespace klhr

@@ -583,5 +583,7 @@ KLHR_DECLARE_MODEL(ar1)
 KLHR_DECLARE_MODEL(ark)
 KLHR_DECLARE_MODEL(rosenbrock)
 KLHR_DECLARE_MODEL(earnings)
+KLHR_DECLARE_MODEL(eight_schools_nc)
+KLHR_DECLARE_MODEL(eight_schools_c)
 
 }  // namespace klhr
