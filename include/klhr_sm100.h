@@ -46,7 +46,9 @@ enum {
                                         w = 1/sigma^2; dim = J + 2, order [theta_trans, mu, log tau] */
     KLHR_MODEL_EIGHT_SCHOOLS_C = 9,  /* posteriordb eight_schools_centered     i0 = J, data0 = [y_1..J | w_1..J],
                                         w = 1/sigma^2; dim = J + 2, order [mu, log tau, theta]       */
-    KLHR_MODEL_COUNT = 10
+    KLHR_MODEL_LOGISTIC_REGRESSION = 10, /* logistic regression  i0 = N >= 0, i1 = K >= 1, data0 = [X (N x (K+1),
+                                            row-major, first column 1) | y_1..N in {0, 1}]; dim = K + 1, order [alpha, beta] */
+    KLHR_MODEL_COUNT = 11
 };
 
 /* Target density descriptor (replaces a bridgestan.StanModel handle, bsmodel.py:10-13). */

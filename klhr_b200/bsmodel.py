@@ -57,6 +57,40 @@ def _eight_schools_data(d):
     return J, y, sigma
 
 
+def _int_at_least(d, key, lo, what):
+    v = d[key]
+    if isinstance(v, bool) or not isinstance(v, (int, np.integer, float, np.floating)) or v != int(v) or v < lo:
+        raise ValueError(f"{what}: {key} must be an integer >= {lo}, got {v!r}")
+    return int(v)
+
+
+def _logistic_regression_data(d):
+    """(N, K, X, y) of the logistic-regression data block, validated: integers N >= 0 and K >= 1, x finite of shape
+    (N, K), y of length N with every entry 0 or 1.  X = [1 | x] is the N x (K + 1) design."""
+    what = "logistic regression"
+    try:
+        N = _int_at_least(d, "N", 0, what)
+        K = _int_at_least(d, "K", 1, what)
+        x = np.asarray(d["x"], dtype=np.float64)
+        y = np.asarray(d["y"], dtype=np.float64)
+    except KeyError as e:
+        raise ValueError(f"{what}: data needs N, K, x[N, K] and y[N] ({e})") from None
+    except (TypeError, ValueError) as e:
+        raise ValueError(f"{what}: x and y must be numeric arrays ({e})") from None
+    if N == 0 and x.size == 0:
+        x = x.reshape(0, K)
+    if x.shape != (N, K):
+        raise ValueError(f"{what}: x must have shape (N, K) = ({N}, {K}), got {x.shape}")
+    if not np.all(np.isfinite(x)):
+        raise ValueError(f"{what}: x must be finite")
+    if y.shape != (N,):
+        raise ValueError(f"{what}: y must have length N = {N}, got shape {y.shape}")
+    if not np.all((y == 0) | (y == 1)):
+        raise ValueError(f"{what}: every y must be 0 or 1")
+    X = np.concatenate([np.ones((N, 1)), x], axis=1)
+    return N, K, X, y
+
+
 class BSModel:
     def __init__(self, stan_file="", data_file="", stepsize=1.0, warn=False, data=None, device=None):
         self._stan_file = stan_file
@@ -130,6 +164,9 @@ class BSModel:
         elif n in _EIGHT_SCHOOLS:                    # posteriordb eight_schools_{noncentered,centered}
             J, y, sigma = _eight_schools_data(d)
             h.update(dim=J + 2, i0=J, data0=np.concatenate([y, 1.0 / (sigma * sigma)]))
+        elif n == "logistic_regression":           # y ~ bernoulli_logit(alpha + x * beta)
+            N, K, X, y = _logistic_regression_data(d)
+            h.update(dim=K + 1, i0=N, i1=K, data0=np.concatenate([X.reshape(-1), y]))
         return h
 
     def dim(self):
@@ -238,6 +275,8 @@ class BSModel:
             return [f"theta_trans.{j + 1}" for j in range(h["i0"])] + ["mu", "tau"]
         if self.name == "eight_schools_centered":
             return ["mu", "tau"] + [f"theta.{j + 1}" for j in range(h["i0"])]
+        if self.name == "logistic_regression":
+            return ["alpha"] + [f"beta.{k + 1}" for k in range(h["i1"])]
         return [f"y.{i + 1}" for i in range(h["dim"])]
 
     def Hamiltonian(self, theta, rho):               # bsmodel.py:45-46

@@ -65,6 +65,12 @@ static int check_model(const klhr_model_t* m, ModelParams& mp) {
             if (!m->data0 || m->i0 < 1 || m->dim != m->i0 + 2)
                 return fail(-5, "eight schools: need data0 = [y|w], i0 = J >= 1, dim = J + 2");
             break;
+        case KLHR_MODEL_LOGISTIC_REGRESSION:
+            if (m->i0 < 0) return fail(-5, "logistic regression: i0 = N must be >= 0");
+            if (m->i1 < 1) return fail(-5, "logistic regression: i1 = K must be >= 1");
+            if (m->dim != m->i1 + 1) return fail(-5, "logistic regression: dim must equal i1 + 1 = K + 1");
+            if (!m->data0 && m->i0 > 0) return fail(-5, "logistic regression: need data0 = [X|y] when N > 0");
+            break;
         default: break;
     }
     return 0;
@@ -134,6 +140,7 @@ static int dispatch_chain(const StepArgs& a, int dtype, int family, bool replay,
         case KLHR_MODEL_EARNINGS: return launch_chain_earnings(a, dtype, family, replay, st, info);
         case KLHR_MODEL_EIGHT_SCHOOLS_NC: return launch_chain_eight_schools_nc(a, dtype, family, replay, st, info);
         case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_chain_eight_schools_c(a, dtype, family, replay, st, info);
+        case KLHR_MODEL_LOGISTIC_REGRESSION: return launch_chain_logistic_regression(a, dtype, family, replay, st, info);
     }
     return fail(-2, "unknown model id");
 }
@@ -155,6 +162,7 @@ static int dispatch_step(const StepArgs& a, int dtype, int family, bool replay, 
         case KLHR_MODEL_EARNINGS: return launch_step_earnings(a, dtype, family, replay, accum, st, info);
         case KLHR_MODEL_EIGHT_SCHOOLS_NC: return launch_step_eight_schools_nc(a, dtype, family, replay, accum, st, info);
         case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_step_eight_schools_c(a, dtype, family, replay, accum, st, info);
+        case KLHR_MODEL_LOGISTIC_REGRESSION: return launch_step_logistic_regression(a, dtype, family, replay, accum, st, info);
     }
     return fail(-2, "unknown model id");
 }
@@ -299,6 +307,7 @@ int klhr_model_eval(const klhr_model_t* model, int dtype, const void* theta_dev,
         case KLHR_MODEL_EARNINGS: e = launch_eval_earnings(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
         case KLHR_MODEL_EIGHT_SCHOOLS_NC: e = launch_eval_eight_schools_nc(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
         case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_eval_eight_schools_c(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
+        case KLHR_MODEL_LOGISTIC_REGRESSION: e = launch_eval_logistic_regression(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
     }
     return cuda_fail(e, "klhr_model_eval");
 }
@@ -409,6 +418,7 @@ int klhr_mh_run(const klhr_model_t* model, int dtype, void* theta_dev, double st
         case KLHR_MODEL_EARNINGS: e = launch_mh_earnings(a, dtype, st); break;
         case KLHR_MODEL_EIGHT_SCHOOLS_NC: e = launch_mh_eight_schools_nc(a, dtype, st); break;
         case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_mh_eight_schools_c(a, dtype, st); break;
+        case KLHR_MODEL_LOGISTIC_REGRESSION: e = launch_mh_logistic_regression(a, dtype, st); break;
     }
     return cuda_fail(e, "klhr_mh_run");
 }
@@ -434,6 +444,7 @@ static int dispatch_slice(const SliceArgs& a, int dtype, bool replay, cudaStream
         case KLHR_MODEL_EARNINGS: return launch_slice_earnings(a, dtype, replay, st);
         case KLHR_MODEL_EIGHT_SCHOOLS_NC: return launch_slice_eight_schools_nc(a, dtype, replay, st);
         case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_slice_eight_schools_c(a, dtype, replay, st);
+        case KLHR_MODEL_LOGISTIC_REGRESSION: return launch_slice_logistic_regression(a, dtype, replay, st);
     }
     return -2;
 }
@@ -520,6 +531,7 @@ int klhr_kl_eval(const klhr_model_t* model, const klhr_fit_t* fit, int dtype, co
         case KLHR_MODEL_EARNINGS: e = launch_kl_earnings(a, dtype, fit->family, st); break;
         case KLHR_MODEL_EIGHT_SCHOOLS_NC: e = launch_kl_eight_schools_nc(a, dtype, fit->family, st); break;
         case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_kl_eight_schools_c(a, dtype, fit->family, st); break;
+        case KLHR_MODEL_LOGISTIC_REGRESSION: e = launch_kl_logistic_regression(a, dtype, fit->family, st); break;
     }
     return cuda_fail(e, "klhr_kl_eval");
 }

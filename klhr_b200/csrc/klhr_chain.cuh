@@ -237,7 +237,10 @@ __global__ void __launch_bounds__(kWarp, KLHR_CHAIN_MINCTAS) chain_kernel(const 
                 R* g = reinterpret_cast<R*>(a.tr.rho) + ((long long)step * a.B + c) * D;
                 for (int i = j; i < D; i += kOct) g[i] = rh[i];
             }
-            const typename Model::Coef cf = Model::setup(th_s, rh, j, om, a.mp);
+            // th_s is the next pass's staging row: a model whose Coef keeps its rows reads the chain's global row,
+            // which holds the same values (written above, ordered by the __syncwarp) and stays put through the fit
+            const R* th_set = CoefKeepsRows<Model>::value ? row : th_s;
+            const typename Model::Coef cf = Model::setup(th_set, rh, j, om, a.mp);
             if (j == p) my_cf = cf;
             __syncwarp(om);                               // th_s is reused by the next pass
         }
@@ -380,5 +383,6 @@ KLHR_DECLARE_MODEL_CHAIN(rosenbrock)
 KLHR_DECLARE_MODEL_CHAIN(earnings)
 KLHR_DECLARE_MODEL_CHAIN(eight_schools_nc)
 KLHR_DECLARE_MODEL_CHAIN(eight_schools_c)
+KLHR_DECLARE_MODEL_CHAIN(logistic_regression)
 
 }  // namespace klhr

@@ -146,5 +146,6 @@ KLHR_DECLARE_MODEL_MH(rosenbrock)
 KLHR_DECLARE_MODEL_MH(earnings)
 KLHR_DECLARE_MODEL_MH(eight_schools_nc)
 KLHR_DECLARE_MODEL_MH(eight_schools_c)
+KLHR_DECLARE_MODEL_MH(logistic_regression)
 
 }  // namespace klhr

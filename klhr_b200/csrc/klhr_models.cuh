@@ -6,7 +6,8 @@
 //                                           memory), result uniform across the 8 lanes; GS = 1 one thread
 //                                           (lane = 0), no shuffles -- the chain kernel's D-phase for small D;
 //   eval(coef, y) -> Jet                    O(1): l(y) - l(0), l'(y), l''(y) of the line
-//                                           restriction l(y) = lp(theta + y rho);
+//                                           restriction l(y) = lp(theta + y rho) (logistic regression: O(N D),
+//                                           a sum over the observations);
 //   lp_grad(th, g, lane, mask, mp) -> lp    full-D log density and gradient (the
 //                                           log_density[_gradient] API, bsmodel.py:15-30).
 // The reference evaluates lp at every quadrature node through the full D-vector
@@ -23,6 +24,13 @@ namespace klhr {
     __device__ static __forceinline__ Jet<R> eval_clip(const Coef& c, R y, const ClipCtx<R>& cc, R& l1c) {             \
         return eval_clip_generic<R, Self>(c, y, cc, l1c);                                                             \
     }
+
+// A model whose Coef keeps the theta / rho row pointers handed to setup (its eval walks the rows: LogisticRegression)
+// declares kCoefKeepsRows = true.  Those rows must stay valid through the fit, so a kernel whose staged theta row is
+// reused before the fit ends hands such a model the chain's own row instead (klhr_chain.cuh, octet D-phase).
+template <typename M, typename = void> struct CoefKeepsRows { static constexpr bool value = false; };
+template <typename M>
+struct CoefKeepsRows<M, decltype((void)M::kCoefKeepsRows)> { static constexpr bool value = M::kCoefKeepsRows; };
 
 struct ModelParams {
     int id;            // KLHR_MODEL_*
@@ -708,6 +716,114 @@ struct EightSchoolsC {
             g[1] = -R(2) * s.sg + R(1 - J) + em2 * sd2;
         }
         return -mu * mu * R(1.0 / 50.0) - s.sp + R(1 - J) * u - R(0.5) * em2 * sd2 - R(0.5) * lik;
+    }
+};
+
+// ------------------------------------------------------------------ logistic regression (a sum over observations)
+// ---- Bayesian logistic regression   params [alpha, beta_1..K], D = K + 1
+//   data { int<lower=0> N; int<lower=1> K; matrix[N, K] x; array[N] int<lower=0, upper=1> y; }
+//   parameters { real alpha; vector[K] beta; }
+//   model { alpha ~ normal(0, 2.5); beta ~ normal(0, 2.5); y ~ bernoulli_logit(alpha + x * beta); }
+// Data: i0 = N (>= 0), i1 = K, data0 = [X (N x D row-major, X[i][0] = 1) | y (N)] in R.
+// lp = -|theta|^2 / 12.5 + sum_i (y_i eta_i - softplus(eta_i)),  eta = X theta.
+//
+// The restriction to the line theta + t rho has no O(1) form: with a = X theta and b = X rho,
+// l(t) = -(|theta|^2 + 2 t theta.rho + t^2 rho.rho) / 12.5 + sum_i (y_i (a_i + t b_i) - softplus(a_i + t b_i)).
+// Storing a and b would cost O(N) memory per chain.  eval recomputes both dot products of every row instead (2 D FMAs,
+// one exp, one log1p per observation), so the chain state stays O(D) and every kernel runs the model unchanged.  X is
+// shared by all chains and the lanes of a warp read the same row at the same time: broadcast loads from L1 / L2.
+// So Coef keeps pointers to the chain's theta and rho rows, which must stay valid through the fit (kCoefKeepsRows).
+// softplus is formed as max(z, 0) + log1p(e^-|z|) (softplus_q): no |eta| overflows in fp32 or fp64.
+template <typename R>
+struct LogisticRegression {
+    using Self = LogisticRegression<R>;
+    static constexpr bool kDenseCta = false;
+    static constexpr bool kCoefKeepsRows = true;
+    struct Coef { const R* th; const R* rh; const R* X; const R* y; int N, D; R tr, rr, l0; };
+    __device__ static __forceinline__ const R* X_(const ModelParams& mp) { return reinterpret_cast<const R*>(mp.p0); }
+    template <int GS = kOct>
+    __device__ static Coef setup(const R* th, const R* rh, int lane, unsigned m, const ModelParams& mp) {
+        Coef c;
+        c.th = th; c.rh = rh; c.N = mp.i0; c.D = mp.D;
+        c.X = X_(mp);
+        c.y = c.X + (size_t)c.N * c.D;
+        R tr = 0, rr = 0, l0 = 0;
+        for (int k = lane; k < c.D; k += GS) {
+            tr += th[k] * rh[k];
+            rr += rh[k] * rh[k];
+        }
+        for (int i = lane; i < c.N; i += GS) {         // the likelihood at t = 0
+            const R* x = c.X + (size_t)i * c.D;
+            R a = 0;
+            for (int k = 0; k < c.D; ++k) a += __ldg(x + k) * th[k];
+            const Softplus<R> s = softplus_q(a, r_exp(-r_abs(a)));
+            l0 += __ldg(c.y + i) * a - s.sp;
+        }
+        c.tr = grp_sum<GS>(tr, m);
+        c.rr = grp_sum<GS>(rr, m);
+        c.l0 = grp_sum<GS>(l0, m);
+        return c;
+    }
+    __device__ static __forceinline__ Jet<R> eval(const Coef& c, R t) {
+        R l = 0, l1 = 0, l2 = 0;
+        const R* x = c.X;
+        for (int i = 0; i < c.N; ++i, x += c.D) {
+            R a = 0, b = 0;
+            for (int k = 0; k < c.D; ++k) {
+                const R xk = __ldg(x + k);
+                a += xk * c.th[k];
+                b += xk * c.rh[k];
+            }
+            const R eta = a + t * b;
+            const Softplus<R> s = softplus_q(eta, r_exp(-r_abs(eta)));
+            const R yi = __ldg(c.y + i);
+            l += yi * eta - s.sp;
+            l1 += b * (yi - s.sg);
+            l2 -= b * b * s.sg1;
+        }
+        return jet_guard<R>(l - c.l0 - t * (R(2) * c.tr + t * c.rr) * R(1.0 / 12.5),
+                            l1 - (c.tr + t * c.rr) * R(1.0 / 6.25), l2 - c.rr * R(1.0 / 6.25));
+    }
+    KLHR_DEFAULT_EVAL_CLIP
+    template <int G = kOct>
+    __device__ static R lp_grad(const R* th, R* g, int lane, unsigned m, const ModelParams& mp) {
+        const int N = mp.i0, D = mp.D;
+        const R* X = X_(mp);
+        const R* yv = X + (size_t)N * D;
+        R acc = 0;
+        for (int k = lane; k < D; k += G) {
+            acc -= th[k] * th[k] * R(1.0 / 12.5);
+            if (g) g[k] = -th[k] * R(1.0 / 6.25);
+        }
+        // observations in groups of G, one per lane; then every lane adds x_ik r_i of the whole group to the gradient
+        // components it owns (k = lane mod G), with r_i = y_i - sigma(eta_i) broadcast from the lane that formed it
+        for (int i0 = 0; i0 < N; i0 += G) {
+            const int i = i0 + lane;
+            R r = 0;
+            if (i < N) {
+                const R* x = X + (size_t)i * D;
+                R a = 0;
+                for (int k = 0; k < D; ++k) a += __ldg(x + k) * th[k];
+                const Softplus<R> s = softplus_q(a, r_exp(-r_abs(a)));
+                const R yi = __ldg(yv + i);
+                acc += yi * a - s.sp;
+                r = yi - s.sg;
+            }
+            if (g) {
+                R rl[G];
+#pragma unroll
+                for (int l = 0; l < G; ++l) rl[l] = G == 1 ? r : __shfl_sync(m, r, l, kOct);
+                const int nl = N - i0 < G ? N - i0 : G;
+                for (int k = lane; k < D; k += G) {
+                    R s = 0;
+#pragma unroll
+                    for (int l = 0; l < G; ++l)
+                        if (l < nl) s += __ldg(X + (size_t)(i0 + l) * D + k) * rl[l];
+                    g[k] += s;
+                }
+            }
+        }
+        return grp_sum<G>(acc, m);
     }
 };
 

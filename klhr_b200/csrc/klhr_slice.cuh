@@ -235,5 +235,6 @@ KLHR_DECLARE_MODEL_SLICE(rosenbrock)
 KLHR_DECLARE_MODEL_SLICE(earnings)
 KLHR_DECLARE_MODEL_SLICE(eight_schools_nc)
 KLHR_DECLARE_MODEL_SLICE(eight_schools_c)
+KLHR_DECLARE_MODEL_SLICE(logistic_regression)
 
 }  // namespace klhr

@@ -585,5 +585,6 @@ KLHR_DECLARE_MODEL(rosenbrock)
 KLHR_DECLARE_MODEL(earnings)
 KLHR_DECLARE_MODEL(eight_schools_nc)
 KLHR_DECLARE_MODEL(eight_schools_c)
+KLHR_DECLARE_MODEL(logistic_regression)
 
 }  // namespace klhr
