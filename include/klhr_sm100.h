@@ -48,7 +48,9 @@ enum {
                                         w = 1/sigma^2; dim = J + 2, order [mu, log tau, theta]       */
     KLHR_MODEL_LOGISTIC_REGRESSION = 10, /* logistic regression  i0 = N >= 0, i1 = K >= 1, data0 = [X (N x (K+1),
                                             row-major, first column 1) | y_1..N in {0, 1}]; dim = K + 1, order [alpha, beta] */
-    KLHR_MODEL_COUNT = 11
+    KLHR_MODEL_ARMA11 = 11,     /* posteriordb arma11, ARMA(1,1)  i0 = T >= 1, data0 = y_1..T; dim = 4,
+                                   order [mu, a, b, v]: phi = tanh(a/2), theta = tanh(b/2), sigma = e^v */
+    KLHR_MODEL_COUNT = 12
 };
 
 /* Target density descriptor (replaces a bridgestan.StanModel handle, bsmodel.py:10-13). */

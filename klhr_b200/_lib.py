@@ -20,7 +20,7 @@ ABI_VERSION = 4
 
 MODEL_IDS = {"normal": 0, "ill-normal": 1, "funnel": 2, "corr-normal": 3, "ar1": 4, "arK": 5,
              "rosenbrock": 6, "earnings": 7, "eight_schools_noncentered": 8, "eight_schools_centered": 9,
-             "logistic_regression": 10}
+             "logistic_regression": 10, "arma11": 11}
 
 
 class ModelDesc(C.Structure):

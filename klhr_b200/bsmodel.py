@@ -91,6 +91,23 @@ def _logistic_regression_data(d):
     return N, K, X, y
 
 
+def _arma11_data(d):
+    """(T, y) of the ARMA(1,1) data block, validated: an integer T >= 1 and y finite of length T."""
+    what = "arma11"
+    try:
+        T = _int_at_least(d, "T", 1, what)
+        y = np.asarray(d["y"], dtype=np.float64)
+    except KeyError as e:
+        raise ValueError(f"{what}: data needs T and y[T] ({e})") from None
+    except (TypeError, ValueError) as e:
+        raise ValueError(f"{what}: y must be a numeric array ({e})") from None
+    if y.shape != (T,):
+        raise ValueError(f"{what}: y must have length T = {T}, got shape {y.shape}")
+    if not np.all(np.isfinite(y)):
+        raise ValueError(f"{what}: y must be finite")
+    return T, y
+
+
 class BSModel:
     def __init__(self, stan_file="", data_file="", stepsize=1.0, warn=False, data=None, device=None):
         self._stan_file = stan_file
@@ -167,6 +184,9 @@ class BSModel:
         elif n == "logistic_regression":           # y ~ bernoulli_logit(alpha + x * beta)
             N, K, X, y = _logistic_regression_data(d)
             h.update(dim=K + 1, i0=N, i1=K, data0=np.concatenate([X.reshape(-1), y]))
+        elif n == "arma11":                          # posteriordb arma11, ARMA(1,1)
+            T, y = _arma11_data(d)
+            h.update(dim=4, i0=T, data0=y)
         return h
 
     def dim(self):
@@ -244,6 +264,13 @@ class BSModel:
         if self.name in _EIGHT_SCHOOLS:              # tau = exp(u)
             k = self._tau_index()
             out[..., k] = torch.exp(out[..., k]) if torch.is_tensor(out) else np.exp(out[..., k])
+        if self.name == "arma11":                    # phi, theta = tanh(a / 2), tanh(b / 2); sigma = exp(v)
+            if torch.is_tensor(out):
+                out[..., 1:3] = torch.tanh(0.5 * out[..., 1:3])
+                out[..., 3] = torch.exp(out[..., 3])
+            else:
+                out[..., 1:3] = np.tanh(0.5 * out[..., 1:3])
+                out[..., 3] = np.exp(out[..., 3])
         return out
 
     def unconstrain(self, theta):
@@ -255,6 +282,13 @@ class BSModel:
         if self.name in _EIGHT_SCHOOLS:
             k = self._tau_index()
             out[..., k] = torch.log(out[..., k]) if torch.is_tensor(out) else np.log(out[..., k])
+        if self.name == "arma11":
+            if torch.is_tensor(out):
+                out[..., 1:3] = 2.0 * torch.atanh(out[..., 1:3])
+                out[..., 3] = torch.log(out[..., 3])
+            else:
+                out[..., 1:3] = 2.0 * np.arctanh(out[..., 1:3])
+                out[..., 3] = np.log(out[..., 3])
         return out
 
     def _tau_index(self):
@@ -277,6 +311,8 @@ class BSModel:
             return ["mu", "tau"] + [f"theta.{j + 1}" for j in range(h["i0"])]
         if self.name == "logistic_regression":
             return ["alpha"] + [f"beta.{k + 1}" for k in range(h["i1"])]
+        if self.name == "arma11":
+            return ["mu", "phi", "theta", "sigma"]
         return [f"y.{i + 1}" for i in range(h["dim"])]
 
     def Hamiltonian(self, theta, rho):               # bsmodel.py:45-46

@@ -71,6 +71,11 @@ static int check_model(const klhr_model_t* m, ModelParams& mp) {
             if (m->dim != m->i1 + 1) return fail(-5, "logistic regression: dim must equal i1 + 1 = K + 1");
             if (!m->data0 && m->i0 > 0) return fail(-5, "logistic regression: need data0 = [X|y] when N > 0");
             break;
+        case KLHR_MODEL_ARMA11:
+            if (m->i0 < 1) return fail(-5, "arma11: i0 = T must be >= 1");
+            if (m->dim != 4) return fail(-5, "arma11: dim must be 4 ([mu, a, b, v])");
+            if (!m->data0) return fail(-5, "arma11: need data0 = y[T]");
+            break;
         default: break;
     }
     return 0;
@@ -141,6 +146,7 @@ static int dispatch_chain(const StepArgs& a, int dtype, int family, bool replay,
         case KLHR_MODEL_EIGHT_SCHOOLS_NC: return launch_chain_eight_schools_nc(a, dtype, family, replay, st, info);
         case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_chain_eight_schools_c(a, dtype, family, replay, st, info);
         case KLHR_MODEL_LOGISTIC_REGRESSION: return launch_chain_logistic_regression(a, dtype, family, replay, st, info);
+        case KLHR_MODEL_ARMA11: return launch_chain_arma11(a, dtype, family, replay, st, info);
     }
     return fail(-2, "unknown model id");
 }
@@ -163,6 +169,7 @@ static int dispatch_step(const StepArgs& a, int dtype, int family, bool replay, 
         case KLHR_MODEL_EIGHT_SCHOOLS_NC: return launch_step_eight_schools_nc(a, dtype, family, replay, accum, st, info);
         case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_step_eight_schools_c(a, dtype, family, replay, accum, st, info);
         case KLHR_MODEL_LOGISTIC_REGRESSION: return launch_step_logistic_regression(a, dtype, family, replay, accum, st, info);
+        case KLHR_MODEL_ARMA11: return launch_step_arma11(a, dtype, family, replay, accum, st, info);
     }
     return fail(-2, "unknown model id");
 }
@@ -308,6 +315,7 @@ int klhr_model_eval(const klhr_model_t* model, int dtype, const void* theta_dev,
         case KLHR_MODEL_EIGHT_SCHOOLS_NC: e = launch_eval_eight_schools_nc(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
         case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_eval_eight_schools_c(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
         case KLHR_MODEL_LOGISTIC_REGRESSION: e = launch_eval_logistic_regression(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
+        case KLHR_MODEL_ARMA11: e = launch_eval_arma11(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
     }
     return cuda_fail(e, "klhr_model_eval");
 }
@@ -419,6 +427,7 @@ int klhr_mh_run(const klhr_model_t* model, int dtype, void* theta_dev, double st
         case KLHR_MODEL_EIGHT_SCHOOLS_NC: e = launch_mh_eight_schools_nc(a, dtype, st); break;
         case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_mh_eight_schools_c(a, dtype, st); break;
         case KLHR_MODEL_LOGISTIC_REGRESSION: e = launch_mh_logistic_regression(a, dtype, st); break;
+        case KLHR_MODEL_ARMA11: e = launch_mh_arma11(a, dtype, st); break;
     }
     return cuda_fail(e, "klhr_mh_run");
 }
@@ -445,6 +454,7 @@ static int dispatch_slice(const SliceArgs& a, int dtype, bool replay, cudaStream
         case KLHR_MODEL_EIGHT_SCHOOLS_NC: return launch_slice_eight_schools_nc(a, dtype, replay, st);
         case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_slice_eight_schools_c(a, dtype, replay, st);
         case KLHR_MODEL_LOGISTIC_REGRESSION: return launch_slice_logistic_regression(a, dtype, replay, st);
+        case KLHR_MODEL_ARMA11: return launch_slice_arma11(a, dtype, replay, st);
     }
     return -2;
 }
@@ -532,6 +542,7 @@ int klhr_kl_eval(const klhr_model_t* model, const klhr_fit_t* fit, int dtype, co
         case KLHR_MODEL_EIGHT_SCHOOLS_NC: e = launch_kl_eight_schools_nc(a, dtype, fit->family, st); break;
         case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_kl_eight_schools_c(a, dtype, fit->family, st); break;
         case KLHR_MODEL_LOGISTIC_REGRESSION: e = launch_kl_logistic_regression(a, dtype, fit->family, st); break;
+        case KLHR_MODEL_ARMA11: e = launch_kl_arma11(a, dtype, fit->family, st); break;
     }
     return cuda_fail(e, "klhr_kl_eval");
 }

@@ -384,5 +384,6 @@ KLHR_DECLARE_MODEL_CHAIN(earnings)
 KLHR_DECLARE_MODEL_CHAIN(eight_schools_nc)
 KLHR_DECLARE_MODEL_CHAIN(eight_schools_c)
 KLHR_DECLARE_MODEL_CHAIN(logistic_regression)
+KLHR_DECLARE_MODEL_CHAIN(arma11)
 
 }  // namespace klhr

@@ -147,5 +147,6 @@ KLHR_DECLARE_MODEL_MH(earnings)
 KLHR_DECLARE_MODEL_MH(eight_schools_nc)
 KLHR_DECLARE_MODEL_MH(eight_schools_c)
 KLHR_DECLARE_MODEL_MH(logistic_regression)
+KLHR_DECLARE_MODEL_MH(arma11)
 
 }  // namespace klhr

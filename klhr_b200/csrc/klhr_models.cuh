@@ -827,4 +827,136 @@ struct LogisticRegression {
     }
 };
 
+// ------------------------------------------------------------------ ARMA(1,1) (a recursion over time)
+// ---- posteriordb arma11 (Stan User's Guide ARMA(1,1))   params [mu, a, b, v], D = 4
+//   data { int<lower=1> T; array[T] real y; }
+//   parameters { real mu; real<lower=-1, upper=1> phi; real<lower=-1, upper=1> theta; real<lower=0> sigma; }
+//   model {
+//     vector[T] nu; vector[T] err;
+//     nu[1] = mu + phi * mu; err[1] = y[1] - nu[1];
+//     for (t in 2:T) { nu[t] = mu + phi * y[t - 1] + theta * err[t - 1]; err[t] = y[t] - nu[t]; }
+//     mu ~ normal(0, 10); phi ~ normal(0, 2); theta ~ normal(0, 2); sigma ~ cauchy(0, 5); err ~ normal(0, sigma);
+//   }
+// Data: i0 = T (>= 1), data0 = y (T) in R.  phi = tanh(a / 2), theta = tanh(b / 2) (lub_constrain to (-1, 1)),
+// sigma = e^v.
+// lp = -mu^2/200 - phi^2/8 - theta^2/8 - softplus(2v - log 25) + (1 - T) v - e^{-2v} sum err^2 / 2 + J(a) + J(b),
+// J(u) = log(d phi / du) = log 2 - |u| - 2 log1p(e^-|u|): log(1 - phi^2) would be -inf once phi rounds to +-1
+// (|a| > ~37 in fp64, ~17 in fp32), where the line searches of the fit still visit.
+//
+// err_t(s) along the line is a polynomial of degree t in theta(s): nothing smaller than the T residuals determines
+// l(s), and they cannot be kept per chain.  eval runs the recursion once per evaluation and carries err_t and its first
+// two s-derivatives: about 14 FMAs per observation and no transcendental in the loop; the three exponentials and three
+// log1p sit outside it.  The chain state stays O(D) and every kernel runs the model unchanged.  The recursion does not
+// split over lanes: setup<GS> has every lane run the s = 0 pass (no shuffles, a uniform result) and lp_grad<G> has
+// every lane run the tangent recursions, lane 0 writing g.
+template <typename R>
+struct Arma11 {
+    using Self = Arma11<R>;
+    static constexpr bool kDenseCta = false;
+    struct Coef { R mu0, rmu, a0, ra, b0, rb, v0, rv, l0; const R* y; int T; };
+    __device__ static __forceinline__ const R* y_(const ModelParams& mp) { return reinterpret_cast<const R*>(mp.p0); }
+    // phi = tanh(u / 2), q = (1 - phi^2) / 2 = d phi / du = 2 e^-|u| / (1 + e^-|u|)^2 and J(u) = log q, all from
+    // e = e^-|u| (q is not formed as 1 - phi^2, which cancels to 0 where q is still a normal number)
+    struct Bounded { R phi, q, J; };
+    static constexpr double kLn2 = 0.6931471805599453;
+    __device__ static __forceinline__ Bounded bounded(R u) {
+        const R e = r_exp(-r_abs(u));
+        const R inv = R(1) / (R(1) + e);
+        const R p = (R(1) - e) * inv;
+        Bounded b;
+        b.phi = u < R(0) ? -p : p;
+        b.q = R(2) * e * inv * inv;
+        b.J = R(kLn2) - r_abs(u) - R(2) * r_log1p(e);
+        return b;
+    }
+    // l(s) = lp(theta + s rho) (not differenced) and its first two s-derivatives
+    __device__ static __forceinline__ Jet<R> line(const Coef& c, R s) {
+        const R mu = c.mu0 + s * c.rmu, v = c.v0 + s * c.rv;
+        const Bounded A = bounded(c.a0 + s * c.ra), B = bounded(c.b0 + s * c.rb);
+        const R ph = A.phi, ph1 = c.ra * A.q, ph2 = -c.ra * c.ra * A.phi * A.q;
+        const R th = B.phi, th1 = c.rb * B.q, th2 = -c.rb * c.rb * B.phi * B.q;
+        // t = 1: err_0 = 0, c_1 = y_1 - mu (1 + phi)
+        R yp = __ldg(c.y);
+        R e = yp - mu * (R(1) + ph);
+        R e1 = -c.rmu * (R(1) + ph) - mu * ph1;
+        R e2 = -R(2) * c.rmu * ph1 - mu * ph2;
+        R E0 = e * e, E1 = e * e1, E2 = e1 * e1 + e * e2;
+        const R th1x2 = R(2) * th1;
+        for (int t = 1; t < c.T; ++t) {
+            const R yt = __ldg(c.y + t);
+            const R n = (yt - mu) - ph * yp - th * e;
+            const R n1 = -c.rmu - ph1 * yp - th1 * e - th * e1;
+            const R n2 = -ph2 * yp - th2 * e - th1x2 * e1 - th * e2;
+            e = n; e1 = n1; e2 = n2;
+            E0 += e * e;
+            E1 += e * e1;
+            E2 += e1 * e1 + e * e2;
+            yp = yt;
+        }
+        const R em2 = r_exp(-R(2) * v);
+        const R z = R(2) * v - R(kLog25);
+        const Softplus<R> sp = softplus_q(z, z >= R(0) ? R(25) * em2 : R(1) / (R(25) * em2));
+        const R omt = R(1 - c.T);
+        Jet<R> j;
+        j.l = -mu * mu * R(1.0 / 200.0) - (ph * ph + th * th) * R(0.125) - sp.sp + omt * v - R(0.5) * em2 * E0 + A.J + B.J;
+        j.l1 = -mu * c.rmu * R(0.01) - (ph * ph1 + th * th1) * R(0.25) - R(2) * c.rv * sp.sg + omt * c.rv
+               - em2 * (E1 - c.rv * E0) - c.ra * A.phi - c.rb * B.phi;
+        j.l2 = -c.rmu * c.rmu * R(0.01) - (ph1 * ph1 + ph * ph2 + th1 * th1 + th * th2) * R(0.25)
+               - R(4) * c.rv * c.rv * sp.sg1 - em2 * (R(2) * c.rv * c.rv * E0 - R(4) * c.rv * E1 + E2)
+               - c.ra * c.ra * A.q - c.rb * c.rb * B.q;
+        return j;
+    }
+    template <int GS = kOct>
+    __device__ static Coef setup(const R* th, const R* rh, int lane, unsigned m, const ModelParams& mp) {
+        Coef c;
+        c.mu0 = th[0]; c.a0 = th[1]; c.b0 = th[2]; c.v0 = th[3];
+        c.rmu = rh[0]; c.ra = rh[1]; c.rb = rh[2]; c.rv = rh[3];
+        c.y = y_(mp);
+        c.T = mp.i0;
+        c.l0 = 0;
+        c.l0 = line(c, R(0)).l;
+        return c;
+    }
+    __device__ static __forceinline__ Jet<R> eval(const Coef& c, R s) {
+        const Jet<R> j = line(c, s);
+        return jet_guard<R>(j.l - c.l0, j.l1, j.l2);
+    }
+    KLHR_DEFAULT_EVAL_CLIP
+    // forward-mode tangents of err_t in mu, a and b: gm_t = -1 - theta gm_{t-1}, ga_t = -phi_a y_{t-1} - theta ga_{t-1},
+    // gb_t = -theta_b err_{t-1} - theta gb_{t-1} (t = 1: -(1 + phi), -mu phi_a, 0); d/dv in closed form
+    template <int G = kOct>
+    __device__ static R lp_grad(const R* th, R* g, int lane, unsigned m, const ModelParams& mp) {
+        const int T = mp.i0;
+        const R* y = y_(mp);
+        const R mu = th[0], v = th[3];
+        const Bounded A = bounded(th[1]), B = bounded(th[2]);
+        const R ph = A.phi, tt = B.phi;
+        R yp = __ldg(y);
+        R e = yp - mu * (R(1) + ph);
+        R gm = -(R(1) + ph), ga = -mu * A.q, gb = 0;
+        R E0 = e * e, Sm = e * gm, Sa = e * ga, Sb = 0;
+        for (int t = 1; t < T; ++t) {
+            const R yt = __ldg(y + t);
+            const R n = (yt - mu) - ph * yp - tt * e;
+            gb = -B.q * e - tt * gb;
+            gm = -R(1) - tt * gm;
+            ga = -A.q * yp - tt * ga;
+            e = n;
+            E0 += e * e; Sm += e * gm; Sa += e * ga; Sb += e * gb;
+            yp = yt;
+        }
+        const R em2 = r_exp(-R(2) * v);
+        const R z = R(2) * v - R(kLog25);
+        const Softplus<R> sp = softplus_q(z, z >= R(0) ? R(25) * em2 : R(1) / (R(25) * em2));
+        if (g && lane == 0) {
+            g[0] = -mu * R(0.01) - em2 * Sm;
+            g[1] = -ph * A.q * R(0.25) - ph - em2 * Sa;
+            g[2] = -tt * B.q * R(0.25) - tt - em2 * Sb;
+            g[3] = -R(2) * sp.sg + R(1 - T) + em2 * E0;
+        }
+        return -mu * mu * R(1.0 / 200.0) - (ph * ph + tt * tt) * R(0.125) - sp.sp + R(1 - T) * v - R(0.5) * em2 * E0
+               + A.J + B.J;
+    }
+};
+
 }  // namespace klhr

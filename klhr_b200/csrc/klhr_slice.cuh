@@ -236,5 +236,6 @@ KLHR_DECLARE_MODEL_SLICE(earnings)
 KLHR_DECLARE_MODEL_SLICE(eight_schools_nc)
 KLHR_DECLARE_MODEL_SLICE(eight_schools_c)
 KLHR_DECLARE_MODEL_SLICE(logistic_regression)
+KLHR_DECLARE_MODEL_SLICE(arma11)
 
 }  // namespace klhr

@@ -586,5 +586,6 @@ KLHR_DECLARE_MODEL(earnings)
 KLHR_DECLARE_MODEL(eight_schools_nc)
 KLHR_DECLARE_MODEL(eight_schools_c)
 KLHR_DECLARE_MODEL(logistic_regression)
+KLHR_DECLARE_MODEL(arma11)
 
 }  // namespace klhr
