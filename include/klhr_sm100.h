@@ -50,7 +50,11 @@ enum {
                                             row-major, first column 1) | y_1..N in {0, 1}]; dim = K + 1, order [alpha, beta] */
     KLHR_MODEL_ARMA11 = 11,     /* posteriordb arma11, ARMA(1,1)  i0 = T >= 1, data0 = y_1..T; dim = 4,
                                    order [mu, a, b, v]: phi = tanh(a/2), theta = tanh(b/2), sigma = e^v */
-    KLHR_MODEL_COUNT = 12
+    KLHR_MODEL_USER = 12,       /* a target compiled from user CUDA source (klhr_b200/csrc/klhr_user.cuh):
+                                   i0 = registry slot (klhr_user_register), i1 = number of data fields F,
+                                   data0 = the fields' values as `dtype` reals, data1 = int64 field table
+                                   (layout in klhr_user.cuh); data0 and data1 are needed when F > 0   */
+    KLHR_MODEL_COUNT = 13
 };
 
 /* Target density descriptor (replaces a bridgestan.StanModel handle, bsmodel.py:10-13). */
@@ -277,6 +281,26 @@ int klhr_philox_eval(const uint32_t* ctr_key_dev, uint32_t* out_dev, int64_t n, 
  * fp32->fp64 promotion, 7 fp64 DMMA m8n8k4) asynchronously on `stream`; the caller times it.  Returns the number of operations the
  * launch issues (thread-level: one FMA = one operation = 2 flop), or < 0 on a bad argument. */
 int64_t klhr_peak_probe(int kind, int64_t iters, int ctas, double* out_dev, void* stream);
+
+/* Launcher table of a user target library (include/klhr_user.h).  The launchers take the library's internal argument
+ * structs by pointer; abi_version and the sizes let klhr_user_register refuse a library built against other
+ * headers.  Every launcher returns 0, a negative klhr code or a cudaError_t, like the built-in targets' launchers. */
+typedef struct klhr_user_table {
+    int32_t abi_version;         /* KLHR_ABI_VERSION the library was built with */
+    int32_t sizeof_step_args, sizeof_slice_args, sizeof_mh_args, sizeof_kl_args, sizeof_model_params;
+    int (*step)(const void* step_args, int dtype, int family, int replay, int accum, void* stream, void* launch_info);
+    int (*chain)(const void* step_args, int dtype, int family, int replay, void* stream, void* launch_info);
+    int (*eval)(const void* model_params, int dtype, const void* theta, void* lp, void* grad, int64_t n_chains,
+                void* stream);
+    int (*kl)(const void* kl_args, int dtype, int family, void* stream);
+    int (*mh)(const void* mh_args, int dtype, void* stream);
+    int (*slice)(const void* slice_args, int dtype, int replay, void* stream);
+} klhr_user_table_t;
+
+/* Registers a user target's launcher table for this process and returns its slot (>= 0), the klhr_model_t.i0 of
+ * KLHR_MODEL_USER descriptors; a table equal to a registered one gets that slot again.  < 0: NULL table or launcher,
+ * ABI version or struct layout mismatch, or a full registry (see klhr_last_error). */
+int klhr_user_register(const klhr_user_table_t* table);
 
 #ifdef __cplusplus
 }

@@ -7,10 +7,11 @@ CUDA kernels behind the C ABI of ``libklhr_sm100.so`` (include/klhr_sm100.h); th
 CPU fallback.
 """
 from .bsmodel import BSModel
+from .cuda_model import CudaModel
 from .engine import (FitConfig, Direction, Trace, SliceConfig, step_replay, run, slice_replay, slice_run, kl_eval,
                      outer_accumulate, outer_scratch, outer_reduce, launch_info, gauss_hermite)
 
-__all__ = ["BSModel", "FitConfig", "Direction", "Trace", "step_replay", "run", "outer_accumulate", "outer_scratch", "outer_reduce",
+__all__ = ["BSModel", "CudaModel", "FitConfig", "Direction", "Trace", "step_replay", "run", "outer_accumulate", "outer_scratch", "outer_reduce",
            "launch_info", "gauss_hermite", "SliceConfig", "slice_replay", "slice_run", "kl_eval"]
 
 try:  # samplers (import kept soft only so that partial checkouts still expose the engine)

@@ -21,6 +21,8 @@ ABI_VERSION = 4
 MODEL_IDS = {"normal": 0, "ill-normal": 1, "funnel": 2, "corr-normal": 3, "ar1": 4, "arK": 5,
              "rosenbrock": 6, "earnings": 7, "eight_schools_noncentered": 8, "eight_schools_centered": 9,
              "logistic_regression": 10, "arma11": 11}
+# targets compiled from user CUDA source (klhr_b200/cuda_model.py); not a Stan program name, so not in MODEL_IDS
+MODEL_USER = 12
 
 
 class ModelDesc(C.Structure):
@@ -61,6 +63,15 @@ class AccumDesc(C.Structure):
                 ("skip_accum_last", C.c_int32), ("thin_offset", C.c_int64)]
 
 
+
+
+class UserTable(C.Structure):
+    _fields_ = [("abi_version", C.c_int32), ("sizeof_step_args", C.c_int32), ("sizeof_slice_args", C.c_int32),
+                ("sizeof_mh_args", C.c_int32), ("sizeof_kl_args", C.c_int32), ("sizeof_model_params", C.c_int32),
+                ("step", C.c_void_p), ("chain", C.c_void_p), ("eval", C.c_void_p), ("kl", C.c_void_p),
+                ("mh", C.c_void_p), ("slice", C.c_void_p)]
+
+
 EXPORTS = {
     "klhr_abi_version": (C.c_int, []),
     "klhr_last_error": (C.c_size_t, [C.c_char_p, C.c_size_t]),
@@ -90,6 +101,7 @@ EXPORTS = {
     "klhr_corr_pack_cholesky": (C.c_int64, [C.c_void_p, C.c_int32, C.c_void_p]),
     "klhr_philox_eval": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "klhr_peak_probe": (C.c_int64, [C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
+    "klhr_user_register": (C.c_int, [C.POINTER(UserTable)]),
     "klhr_launch_info": (C.c_int, [C.POINTER(ModelDesc), C.POINTER(FitDesc), C.c_int, C.c_int, C.c_int,
                                    C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
 }

@@ -1,9 +1,11 @@
 // klhr_b200 -- extern "C" entry points of libklhr_sm100.so (include/klhr_sm100.h).
 // Validation, error strings and dispatch only; the kernels are in klhr_step.cuh and the
 // per-model translation units.
+#include <atomic>
 #include <cstdio>
 #include <cstring>
 #include <cmath>
+#include <mutex>
 #include <string>
 
 #include "klhr_chain.cuh"
@@ -29,6 +31,16 @@ static int cuda_fail(int e, const char* where) {
     }
     return e;
 }
+
+// ------------------------------------------------------------------ user targets
+// Launcher tables of the user target libraries registered in this process (klhr_user_register).  A slot is written
+// once, before the count that publishes it, and never changes, so the dispatchers read it without the lock.
+constexpr int kUserSlots = 64;
+static klhr_user_table_t g_user[kUserSlots];
+static std::atomic<int> g_user_count{0};
+static std::mutex g_user_mutex;
+
+static const klhr_user_table_t& user_table(const ModelParams& mp) { return g_user[mp.i0]; }
 
 static int check_model(const klhr_model_t* m, ModelParams& mp) {
     if (!m) return fail(-1, "model is NULL");
@@ -75,6 +87,13 @@ static int check_model(const klhr_model_t* m, ModelParams& mp) {
             if (m->i0 < 1) return fail(-5, "arma11: i0 = T must be >= 1");
             if (m->dim != 4) return fail(-5, "arma11: dim must be 4 ([mu, a, b, v])");
             if (!m->data0) return fail(-5, "arma11: need data0 = y[T]");
+            break;
+        case KLHR_MODEL_USER:
+            if (m->i0 < 0 || m->i0 >= g_user_count.load(std::memory_order_acquire))
+                return fail(-5, "user target: i0 is not a registered slot (klhr_user_register)");
+            if (m->i1 < 0) return fail(-5, "user target: i1 = number of data fields must be >= 0");
+            if (m->i1 > 0 && (!m->data0 || !m->data1))
+                return fail(-5, "user target: data fields declared (i1 > 0) need data0 = values and data1 = field table");
             break;
         default: break;
     }
@@ -147,6 +166,7 @@ static int dispatch_chain(const StepArgs& a, int dtype, int family, bool replay,
         case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_chain_eight_schools_c(a, dtype, family, replay, st, info);
         case KLHR_MODEL_LOGISTIC_REGRESSION: return launch_chain_logistic_regression(a, dtype, family, replay, st, info);
         case KLHR_MODEL_ARMA11: return launch_chain_arma11(a, dtype, family, replay, st, info);
+        case KLHR_MODEL_USER: return user_table(a.mp).chain(&a, dtype, family, replay, st, info);
     }
     return fail(-2, "unknown model id");
 }
@@ -170,6 +190,7 @@ static int dispatch_step(const StepArgs& a, int dtype, int family, bool replay, 
         case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_step_eight_schools_c(a, dtype, family, replay, accum, st, info);
         case KLHR_MODEL_LOGISTIC_REGRESSION: return launch_step_logistic_regression(a, dtype, family, replay, accum, st, info);
         case KLHR_MODEL_ARMA11: return launch_step_arma11(a, dtype, family, replay, accum, st, info);
+        case KLHR_MODEL_USER: return user_table(a.mp).step(&a, dtype, family, replay, accum, st, info);
     }
     return fail(-2, "unknown model id");
 }
@@ -285,6 +306,26 @@ extern "C" {
 
 int klhr_abi_version(void) { return KLHR_ABI_VERSION; }
 
+int klhr_user_register(const klhr_user_table_t* t) {
+    if (!t) return fail(-1, "klhr_user_register: table is NULL");
+    if (t->abi_version != KLHR_ABI_VERSION)
+        return fail(-17, "klhr_user_register: the user library was built for another ABI version");
+    if (t->sizeof_step_args != (int32_t)sizeof(StepArgs) || t->sizeof_slice_args != (int32_t)sizeof(SliceArgs) ||
+        t->sizeof_mh_args != (int32_t)sizeof(MhArgs) || t->sizeof_kl_args != (int32_t)sizeof(KlArgs) ||
+        t->sizeof_model_params != (int32_t)sizeof(ModelParams))
+        return fail(-17, "klhr_user_register: argument struct layout mismatch (the user library was built against other headers)");
+    if (!t->step || !t->chain || !t->eval || !t->kl || !t->mh || !t->slice)
+        return fail(-1, "klhr_user_register: a launcher of the table is NULL");
+    std::lock_guard<std::mutex> lock(g_user_mutex);
+    const int n = g_user_count.load(std::memory_order_relaxed);
+    for (int k = 0; k < n; ++k)
+        if (std::memcmp(&g_user[k], t, sizeof(*t)) == 0) return k;
+    if (n == kUserSlots) return fail(-18, "klhr_user_register: registry full (64 user targets per process)");
+    g_user[n] = *t;
+    g_user_count.store(n + 1, std::memory_order_release);
+    return n;
+}
+
 size_t klhr_last_error(char* buf, size_t len) {
     if (!buf || len == 0) return g_last_error.size();
     const size_t n = g_last_error.size() < len - 1 ? g_last_error.size() : len - 1;
@@ -316,6 +357,7 @@ int klhr_model_eval(const klhr_model_t* model, int dtype, const void* theta_dev,
         case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_eval_eight_schools_c(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
         case KLHR_MODEL_LOGISTIC_REGRESSION: e = launch_eval_logistic_regression(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
         case KLHR_MODEL_ARMA11: e = launch_eval_arma11(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
+        case KLHR_MODEL_USER: e = user_table(mp).eval(&mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
     }
     return cuda_fail(e, "klhr_model_eval");
 }
@@ -428,6 +470,7 @@ int klhr_mh_run(const klhr_model_t* model, int dtype, void* theta_dev, double st
         case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_mh_eight_schools_c(a, dtype, st); break;
         case KLHR_MODEL_LOGISTIC_REGRESSION: e = launch_mh_logistic_regression(a, dtype, st); break;
         case KLHR_MODEL_ARMA11: e = launch_mh_arma11(a, dtype, st); break;
+        case KLHR_MODEL_USER: e = user_table(a.mp).mh(&a, dtype, st); break;
     }
     return cuda_fail(e, "klhr_mh_run");
 }
@@ -455,6 +498,7 @@ static int dispatch_slice(const SliceArgs& a, int dtype, bool replay, cudaStream
         case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_slice_eight_schools_c(a, dtype, replay, st);
         case KLHR_MODEL_LOGISTIC_REGRESSION: return launch_slice_logistic_regression(a, dtype, replay, st);
         case KLHR_MODEL_ARMA11: return launch_slice_arma11(a, dtype, replay, st);
+        case KLHR_MODEL_USER: return user_table(a.mp).slice(&a, dtype, replay, st);
     }
     return -2;
 }
@@ -543,6 +587,7 @@ int klhr_kl_eval(const klhr_model_t* model, const klhr_fit_t* fit, int dtype, co
         case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_kl_eight_schools_c(a, dtype, fit->family, st); break;
         case KLHR_MODEL_LOGISTIC_REGRESSION: e = launch_kl_logistic_regression(a, dtype, fit->family, st); break;
         case KLHR_MODEL_ARMA11: e = launch_kl_arma11(a, dtype, fit->family, st); break;
+        case KLHR_MODEL_USER: e = user_table(a.mp).kl(&a, dtype, fit->family, st); break;
     }
     return cuda_fail(e, "klhr_kl_eval");
 }
