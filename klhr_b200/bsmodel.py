@@ -19,6 +19,7 @@ from __future__ import annotations
 import ctypes as C
 import json
 from pathlib import Path
+from typing import Callable, NamedTuple
 
 import numpy as np
 import torch
@@ -33,9 +34,6 @@ def _dtype_code(dtype):
         return _DTYPES[dtype]
     except KeyError:
         raise TypeError(f"klhr_b200 computes in float64 or float32, not {dtype}") from None
-
-
-_EIGHT_SCHOOLS = ("eight_schools_noncentered", "eight_schools_centered")
 
 
 def _eight_schools_data(d):
@@ -108,6 +106,125 @@ def _arma11_data(d):
     return T, y
 
 
+# ---------------------------------------------------------------------- one record per Stan program
+# prepare: the data block -> the descriptor fields that differ from the defaults (the program's "transformed data");
+# names: the host fields -> the parameter names; fp64_data: data0 holds sufficient statistics that stay fp64 whatever
+# the arithmetic type (klhr_models.cuh); transforms: (index or slice, kind) of every coordinate whose constrained value
+# is exp(u) ("exp") or tanh(u / 2) ("tanh_half").
+class _Target(NamedTuple):
+    prepare: Callable[[dict], dict]
+    names: Callable[[dict], list]
+    fp64_data: bool = False
+    transforms: tuple = ()
+
+
+def _y_names(h):
+    return [f"y.{i + 1}" for i in range(h["dim"])]
+
+
+def _ill_normal(d):                                  # stan/ill-normal.stan:4-6
+    D = int(d["D"])
+    s = np.arange(1, D + 1, dtype=np.float64) / np.sqrt(float(D))
+    return dict(dim=D, data0=1.0 / (s * s))
+
+
+def _corr_normal(d):                                 # stan/corr-normal.stan:5-13
+    N, rho = int(d["N"]), float(d["rho"])
+    idx = np.arange(N)
+    Sigma = rho ** np.abs(idx[:, None] - idx[None, :])
+    P = np.linalg.inv(Sigma)
+    P = 0.5 * (P + P.T)
+    h = dict(dim=N, data0=P.reshape(-1))
+    if N in (128, 256):
+        # P = L L' (fp64): the dense kernels work with V = L' rho and w = L' theta (csrc/klhr_densek.cuh); L goes
+        # to the device packed in the order the tensor warps consume it (klhr_corr_pack_cholesky)
+        L = np.ascontiguousarray(np.tril(np.linalg.cholesky(P)), dtype=np.float64)
+        lib = _lib.load()
+        n = lib.klhr_corr_pack_cholesky(None, N, None)
+        packed = np.empty(int(n), dtype=np.float64)
+        if lib.klhr_corr_pack_cholesky(L.ctypes.data, N, packed.ctypes.data) != n:
+            raise _lib.KLHRLibraryError(f"klhr_corr_pack_cholesky failed: {_lib.last_error()}")
+        h["data1"] = packed
+    return h
+
+
+def _ar1(d):                                         # stan/ar1.stan:4-7
+    alpha = 0.9
+    return dict(dim=int(d["N"]), s0=alpha, s1=1.0 / (1.0 - alpha * alpha))
+
+
+def _ark(d):                                         # stan/arK.stan:1-20, sufficient statistics
+    K, T = int(d["K"]), int(d["T"])
+    y = np.asarray(d["y"], dtype=np.float64)
+    if y.shape != (T,):
+        raise ValueError("arK: len(y) must equal T")
+    nobs = T - K
+    X = np.empty((nobs, K + 1))
+    X[:, 0] = 1.0
+    for k in range(K):
+        X[:, 1 + k] = y[k:k + nobs]
+    yt = y[K:]
+    pack = np.concatenate([(X.T @ X).reshape(-1), X.T @ yt, [yt @ yt]])
+    return dict(dim=K + 2, i0=K, i1=nobs, data0=pack)
+
+
+def _earnings(d):                                    # stan/earnings.stan:1-17, sufficient statistics
+    e = np.asarray(d["earn"], dtype=np.float64)
+    ht = np.asarray(d["height"], dtype=np.float64)
+    if e.shape != (int(d["N"]),) or ht.shape != e.shape:
+        raise ValueError("earnings: earn and height must have length N")
+    return dict(dim=4, data0=np.array([float(len(e)), e.sum(), ht.sum(), e @ e, e @ ht, ht @ ht]))
+
+
+def _eight_schools(d):                               # posteriordb eight_schools_{noncentered,centered}
+    J, y, sigma = _eight_schools_data(d)
+    return dict(dim=J + 2, i0=J, data0=np.concatenate([y, 1.0 / (sigma * sigma)]))
+
+
+def _logistic_regression(d):                         # y ~ bernoulli_logit(alpha + x * beta)
+    N, K, X, y = _logistic_regression_data(d)
+    return dict(dim=K + 1, i0=N, i1=K, data0=np.concatenate([X.reshape(-1), y]))
+
+
+def _arma11(d):                                      # posteriordb arma11, ARMA(1,1)
+    T, y = _arma11_data(d)
+    return dict(dim=4, i0=T, data0=y)
+
+
+_TARGETS = {
+    "normal": _Target(lambda d: dict(dim=int(d["D"])), _y_names),
+    "ill-normal": _Target(_ill_normal, _y_names),
+    # stan/funnel.stan:4-7
+    "funnel": _Target(lambda d: dict(dim=int(d["D"]) + 1, i0=int(d["D"])),
+                      lambda h: ["double_log_sigma"] + [f"alpha.{i + 1}" for i in range(h["i0"])]),
+    "corr-normal": _Target(_corr_normal, _y_names),
+    "ar1": _Target(_ar1, _y_names),
+    # sigma = exp(u), stan/arK.stan:9
+    "arK": _Target(_ark, lambda h: ["alpha"] + [f"beta.{i + 1}" for i in range(h["i0"])] + ["sigma"],
+                   fp64_data=True, transforms=((-1, "exp"),)),
+    # stan/rosenbrock.stan:4-7
+    "rosenbrock": _Target(lambda d: dict(dim=2 * int(d["D"]), i0=int(d["D"])),
+                          lambda h: ([f"v.{i + 1}" for i in range(h["i0"])] +
+                                     [f"theta.{i + 1}" for i in range(h["i0"])])),
+    # sigma, s > 0, stan/earnings.stan:9-10
+    "earnings": _Target(_earnings, lambda h: ["beta.1", "beta.2", "sigma", "s"],
+                        fp64_data=True, transforms=((slice(2, None), "exp"),)),
+    # [theta_trans, mu, log tau]
+    "eight_schools_noncentered": _Target(
+        _eight_schools, lambda h: [f"theta_trans.{j + 1}" for j in range(h["i0"])] + ["mu", "tau"],
+        transforms=((-1, "exp"),)),
+    # [mu, log tau, theta]
+    "eight_schools_centered": _Target(
+        _eight_schools, lambda h: ["mu", "tau"] + [f"theta.{j + 1}" for j in range(h["i0"])],
+        transforms=((1, "exp"),)),
+    "logistic_regression": _Target(_logistic_regression,
+                                   lambda h: ["alpha"] + [f"beta.{k + 1}" for k in range(h["i1"])]),
+    # [mu, a, b, v]: phi, theta = tanh(a / 2), tanh(b / 2); sigma = exp(v)
+    "arma11": _Target(_arma11, lambda h: ["mu", "phi", "theta", "sigma"],
+                      transforms=((slice(1, 3), "tanh_half"), (3, "exp"))),
+}
+
+
 class BSModel:
     def __init__(self, stan_file="", data_file="", stepsize=1.0, warn=False, data=None, device=None):
         self._stan_file = stan_file
@@ -127,66 +244,8 @@ class BSModel:
 
     # ------------------------------------------------------------------ host-side "transformed data"
     def _prepare_host(self):
-        d, n = self.data, self.name
         h = dict(i0=0, i1=0, s0=0.0, s1=0.0, data0=None, data1=None)
-        if n == "normal":
-            h["dim"] = int(d["D"])
-        elif n == "ill-normal":                      # stan/ill-normal.stan:4-6
-            D = int(d["D"])
-            s = np.arange(1, D + 1, dtype=np.float64) / np.sqrt(float(D))
-            h.update(dim=D, data0=1.0 / (s * s))
-        elif n == "funnel":                          # stan/funnel.stan:4-7
-            h.update(dim=int(d["D"]) + 1, i0=int(d["D"]))
-        elif n == "corr-normal":                     # stan/corr-normal.stan:5-13
-            N, rho = int(d["N"]), float(d["rho"])
-            idx = np.arange(N)
-            Sigma = rho ** np.abs(idx[:, None] - idx[None, :])
-            P = np.linalg.inv(Sigma)
-            P = 0.5 * (P + P.T)
-            h.update(dim=N, data0=P.reshape(-1))
-            if N in (128, 256):
-                # P = L L' (fp64): the dense kernels work with V = L' rho and w = L' theta (csrc/klhr_densek.cuh); L goes
-                # to the device packed in the order the tensor warps consume it (klhr_corr_pack_cholesky)
-                L = np.ascontiguousarray(np.tril(np.linalg.cholesky(P)), dtype=np.float64)
-                lib = _lib.load()
-                n = lib.klhr_corr_pack_cholesky(None, N, None)
-                packed = np.empty(int(n), dtype=np.float64)
-                if lib.klhr_corr_pack_cholesky(L.ctypes.data, N, packed.ctypes.data) != n:
-                    raise _lib.KLHRLibraryError(f"klhr_corr_pack_cholesky failed: {_lib.last_error()}")
-                h["data1"] = packed
-        elif n == "ar1":                             # stan/ar1.stan:4-7
-            alpha = 0.9
-            h.update(dim=int(d["N"]), s0=alpha, s1=1.0 / (1.0 - alpha * alpha))
-        elif n == "arK":                             # stan/arK.stan:1-20, sufficient statistics
-            K, T = int(d["K"]), int(d["T"])
-            y = np.asarray(d["y"], dtype=np.float64)
-            if y.shape != (T,):
-                raise ValueError("arK: len(y) must equal T")
-            nobs = T - K
-            X = np.empty((nobs, K + 1))
-            X[:, 0] = 1.0
-            for k in range(K):
-                X[:, 1 + k] = y[k:k + nobs]
-            yt = y[K:]
-            pack = np.concatenate([(X.T @ X).reshape(-1), X.T @ yt, [yt @ yt]])
-            h.update(dim=K + 2, i0=K, i1=nobs, data0=pack)
-        elif n == "rosenbrock":                      # stan/rosenbrock.stan:4-7
-            h.update(dim=2 * int(d["D"]), i0=int(d["D"]))
-        elif n == "earnings":                        # stan/earnings.stan:1-17, sufficient statistics
-            e = np.asarray(d["earn"], dtype=np.float64)
-            ht = np.asarray(d["height"], dtype=np.float64)
-            if e.shape != (int(d["N"]),) or ht.shape != e.shape:
-                raise ValueError("earnings: earn and height must have length N")
-            h.update(dim=4, data0=np.array([float(len(e)), e.sum(), ht.sum(), e @ e, e @ ht, ht @ ht]))
-        elif n in _EIGHT_SCHOOLS:                    # posteriordb eight_schools_{noncentered,centered}
-            J, y, sigma = _eight_schools_data(d)
-            h.update(dim=J + 2, i0=J, data0=np.concatenate([y, 1.0 / (sigma * sigma)]))
-        elif n == "logistic_regression":           # y ~ bernoulli_logit(alpha + x * beta)
-            N, K, X, y = _logistic_regression_data(d)
-            h.update(dim=K + 1, i0=N, i1=K, data0=np.concatenate([X.reshape(-1), y]))
-        elif n == "arma11":                          # posteriordb arma11, ARMA(1,1)
-            T, y = _arma11_data(d)
-            h.update(dim=4, i0=T, data0=y)
+        h.update(_TARGETS[self.name].prepare(self.data))
         return h
 
     def dim(self):
@@ -202,7 +261,7 @@ class BSModel:
             buf = None
             if h["data0"] is not None:
                 # sufficient statistics (arK, earnings) stay fp64 whatever the arithmetic type (klhr_models.cuh)
-                bt = torch.float64 if self.name in ("arK", "earnings") else dtype
+                bt = torch.float64 if _TARGETS[self.name].fp64_data else dtype
                 buf = torch.as_tensor(h["data0"], dtype=torch.float64).to(device=device, dtype=bt).contiguous()
             buf1 = None
             if h.get("data1") is not None and dtype == torch.float64:
@@ -255,65 +314,25 @@ class BSModel:
         return self._eval(theta, True)
 
     # ------------------------------------------------------------------ transforms / names
-    def constrain(self, theta):
+    def _transform(self, theta, inverse):
         out = theta.clone() if torch.is_tensor(theta) else np.array(theta, dtype=np.float64)
-        if self.name == "arK":                       # sigma = exp(u), stan/arK.stan:9
-            out[..., -1] = torch.exp(out[..., -1]) if torch.is_tensor(out) else np.exp(out[..., -1])
-        if self.name == "earnings":                  # sigma, s > 0, stan/earnings.stan:9-10
-            out[..., 2:] = torch.exp(out[..., 2:]) if torch.is_tensor(out) else np.exp(out[..., 2:])
-        if self.name in _EIGHT_SCHOOLS:              # tau = exp(u)
-            k = self._tau_index()
-            out[..., k] = torch.exp(out[..., k]) if torch.is_tensor(out) else np.exp(out[..., k])
-        if self.name == "arma11":                    # phi, theta = tanh(a / 2), tanh(b / 2); sigma = exp(v)
-            if torch.is_tensor(out):
-                out[..., 1:3] = torch.tanh(0.5 * out[..., 1:3])
-                out[..., 3] = torch.exp(out[..., 3])
-            else:
-                out[..., 1:3] = np.tanh(0.5 * out[..., 1:3])
-                out[..., 3] = np.exp(out[..., 3])
+        xp = torch if torch.is_tensor(out) else np
+        for k, kind in _TARGETS[self.name].transforms:
+            u = out[..., k]
+            if kind == "exp":
+                out[..., k] = xp.log(u) if inverse else xp.exp(u)
+            else:                                    # "tanh_half"
+                out[..., k] = 2.0 * xp.arctanh(u) if inverse else xp.tanh(0.5 * u)
         return out
+
+    def constrain(self, theta):
+        return self._transform(theta, inverse=False)
 
     def unconstrain(self, theta):
-        out = theta.clone() if torch.is_tensor(theta) else np.array(theta, dtype=np.float64)
-        if self.name == "arK":
-            out[..., -1] = torch.log(out[..., -1]) if torch.is_tensor(out) else np.log(out[..., -1])
-        if self.name == "earnings":
-            out[..., 2:] = torch.log(out[..., 2:]) if torch.is_tensor(out) else np.log(out[..., 2:])
-        if self.name in _EIGHT_SCHOOLS:
-            k = self._tau_index()
-            out[..., k] = torch.log(out[..., k]) if torch.is_tensor(out) else np.log(out[..., k])
-        if self.name == "arma11":
-            if torch.is_tensor(out):
-                out[..., 1:3] = 2.0 * torch.atanh(out[..., 1:3])
-                out[..., 3] = torch.log(out[..., 3])
-            else:
-                out[..., 1:3] = 2.0 * np.arctanh(out[..., 1:3])
-                out[..., 3] = np.log(out[..., 3])
-        return out
-
-    def _tau_index(self):
-        """Position of tau (unconstrained: log tau) in the parameter vector of the eight-schools programs."""
-        return self._host["i0"] + 1 if self.name == "eight_schools_noncentered" else 1
+        return self._transform(theta, inverse=True)
 
     def parameter_names(self):
-        h = self._host
-        if self.name == "funnel":
-            return ["double_log_sigma"] + [f"alpha.{i + 1}" for i in range(h["i0"])]
-        if self.name == "arK":
-            return ["alpha"] + [f"beta.{i + 1}" for i in range(h["i0"])] + ["sigma"]
-        if self.name == "earnings":
-            return ["beta.1", "beta.2", "sigma", "s"]
-        if self.name == "rosenbrock":
-            return [f"v.{i + 1}" for i in range(h["i0"])] + [f"theta.{i + 1}" for i in range(h["i0"])]
-        if self.name == "eight_schools_noncentered":
-            return [f"theta_trans.{j + 1}" for j in range(h["i0"])] + ["mu", "tau"]
-        if self.name == "eight_schools_centered":
-            return ["mu", "tau"] + [f"theta.{j + 1}" for j in range(h["i0"])]
-        if self.name == "logistic_regression":
-            return ["alpha"] + [f"beta.{k + 1}" for k in range(h["i1"])]
-        if self.name == "arma11":
-            return ["mu", "phi", "theta", "sigma"]
-        return [f"y.{i + 1}" for i in range(h["dim"])]
+        return _TARGETS[self.name].names(self._host)
 
     def Hamiltonian(self, theta, rho):               # bsmodel.py:45-46
         return -self.log_density(theta) + 0.5 * (rho * rho).sum(-1)

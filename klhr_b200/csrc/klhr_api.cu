@@ -40,7 +40,44 @@ static klhr_user_table_t g_user[kUserSlots];
 static std::atomic<int> g_user_count{0};
 static std::mutex g_user_mutex;
 
-static const klhr_user_table_t& user_table(const ModelParams& mp) { return g_user[mp.i0]; }
+// ------------------------------------------------------------------ built-in targets
+// Launcher tables of the built-in targets (klhr_model_*.cu), indexed by model id.
+extern const klhr_user_table_t kNormalLaunchers, kIllNormalLaunchers, kFunnelLaunchers, kCorrNormalLaunchers,
+    kAr1Launchers, kArkLaunchers, kRosenbrockLaunchers, kEarningsLaunchers, kEightSchoolsNCLaunchers,
+    kEightSchoolsCLaunchers, kLogisticRegressionLaunchers, kArma11Launchers;
+
+struct BuiltinTargets { const klhr_user_table_t* t[KLHR_MODEL_USER]; };
+
+constexpr BuiltinTargets builtin_targets() {
+    BuiltinTargets b{};
+    b.t[KLHR_MODEL_NORMAL] = &kNormalLaunchers;
+    b.t[KLHR_MODEL_ILL_NORMAL] = &kIllNormalLaunchers;
+    b.t[KLHR_MODEL_FUNNEL] = &kFunnelLaunchers;
+    b.t[KLHR_MODEL_CORR_NORMAL] = &kCorrNormalLaunchers;
+    b.t[KLHR_MODEL_AR1] = &kAr1Launchers;
+    b.t[KLHR_MODEL_ARK] = &kArkLaunchers;
+    b.t[KLHR_MODEL_ROSENBROCK] = &kRosenbrockLaunchers;
+    b.t[KLHR_MODEL_EARNINGS] = &kEarningsLaunchers;
+    b.t[KLHR_MODEL_EIGHT_SCHOOLS_NC] = &kEightSchoolsNCLaunchers;
+    b.t[KLHR_MODEL_EIGHT_SCHOOLS_C] = &kEightSchoolsCLaunchers;
+    b.t[KLHR_MODEL_LOGISTIC_REGRESSION] = &kLogisticRegressionLaunchers;
+    b.t[KLHR_MODEL_ARMA11] = &kArma11Launchers;
+    return b;
+}
+
+constexpr BuiltinTargets kBuiltin = builtin_targets();
+
+constexpr bool every_id_has_a_table(const BuiltinTargets& b) {
+    for (const klhr_user_table_t* t : b.t)
+        if (!t) return false;
+    return true;
+}
+static_assert(every_id_has_a_table(kBuiltin), "a model id below KLHR_MODEL_USER has no launcher table");
+
+// The launchers of a descriptor that passed check_model.
+static const klhr_user_table_t& launchers(const ModelParams& mp) {
+    return mp.id == KLHR_MODEL_USER ? g_user[mp.i0] : *kBuiltin.t[mp.id];
+}
 
 static int check_model(const klhr_model_t* m, ModelParams& mp) {
     if (!m) return fail(-1, "model is NULL");
@@ -152,47 +189,13 @@ static bool chain_applies(const StepArgs& a, int dtype, bool replay, bool accum,
            chain_smem_bytes(a, dtype == KLHR_F64 ? 8 : 4, replay) <= 20 * 1024;   // larger D: the octet kernel keeps theta resident
 }
 
-static int dispatch_chain(const StepArgs& a, int dtype, int family, bool replay, cudaStream_t st, LaunchInfo* info) {
-    switch (a.mp.id) {
-        case KLHR_MODEL_NORMAL: return launch_chain_normal(a, dtype, family, replay, st, info);
-        case KLHR_MODEL_ILL_NORMAL: return launch_chain_ill_normal(a, dtype, family, replay, st, info);
-        case KLHR_MODEL_FUNNEL: return launch_chain_funnel(a, dtype, family, replay, st, info);
-        case KLHR_MODEL_CORR_NORMAL: return launch_chain_corr_normal(a, dtype, family, replay, st, info);
-        case KLHR_MODEL_AR1: return launch_chain_ar1(a, dtype, family, replay, st, info);
-        case KLHR_MODEL_ARK: return launch_chain_ark(a, dtype, family, replay, st, info);
-        case KLHR_MODEL_ROSENBROCK: return launch_chain_rosenbrock(a, dtype, family, replay, st, info);
-        case KLHR_MODEL_EARNINGS: return launch_chain_earnings(a, dtype, family, replay, st, info);
-        case KLHR_MODEL_EIGHT_SCHOOLS_NC: return launch_chain_eight_schools_nc(a, dtype, family, replay, st, info);
-        case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_chain_eight_schools_c(a, dtype, family, replay, st, info);
-        case KLHR_MODEL_LOGISTIC_REGRESSION: return launch_chain_logistic_regression(a, dtype, family, replay, st, info);
-        case KLHR_MODEL_ARMA11: return launch_chain_arma11(a, dtype, family, replay, st, info);
-        case KLHR_MODEL_USER: return user_table(a.mp).chain(&a, dtype, family, replay, st, info);
-    }
-    return fail(-2, "unknown model id");
-}
-
 static int dispatch_step(const StepArgs& a, int dtype, int family, bool replay, bool accum, cudaStream_t st,
                          LaunchInfo* info, int flags) {
     if (lane_applies(a, dtype, family, replay, accum, flags)) return launch_lane(a, st, info);
     if (densek_applies(a, dtype, family, replay, accum, flags)) return launch_densek(a, replay, st, info);
     if (tile_applies(a, family, accum, flags)) return launch_tile(a, dtype, replay, st, info);
-    if (chain_applies(a, dtype, replay, accum, flags)) return dispatch_chain(a, dtype, family, replay, st, info);
-    switch (a.mp.id) {
-        case KLHR_MODEL_NORMAL: return launch_step_normal(a, dtype, family, replay, accum, st, info);
-        case KLHR_MODEL_ILL_NORMAL: return launch_step_ill_normal(a, dtype, family, replay, accum, st, info);
-        case KLHR_MODEL_FUNNEL: return launch_step_funnel(a, dtype, family, replay, accum, st, info);
-        case KLHR_MODEL_CORR_NORMAL: return launch_step_corr_normal(a, dtype, family, replay, accum, st, info);
-        case KLHR_MODEL_AR1: return launch_step_ar1(a, dtype, family, replay, accum, st, info);
-        case KLHR_MODEL_ARK: return launch_step_ark(a, dtype, family, replay, accum, st, info);
-        case KLHR_MODEL_ROSENBROCK: return launch_step_rosenbrock(a, dtype, family, replay, accum, st, info);
-        case KLHR_MODEL_EARNINGS: return launch_step_earnings(a, dtype, family, replay, accum, st, info);
-        case KLHR_MODEL_EIGHT_SCHOOLS_NC: return launch_step_eight_schools_nc(a, dtype, family, replay, accum, st, info);
-        case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_step_eight_schools_c(a, dtype, family, replay, accum, st, info);
-        case KLHR_MODEL_LOGISTIC_REGRESSION: return launch_step_logistic_regression(a, dtype, family, replay, accum, st, info);
-        case KLHR_MODEL_ARMA11: return launch_step_arma11(a, dtype, family, replay, accum, st, info);
-        case KLHR_MODEL_USER: return user_table(a.mp).step(&a, dtype, family, replay, accum, st, info);
-    }
-    return fail(-2, "unknown model id");
+    if (chain_applies(a, dtype, replay, accum, flags)) return launchers(a.mp).chain(&a, dtype, family, replay, st, info);
+    return launchers(a.mp).step(&a, dtype, family, replay, accum, st, info);
 }
 
 // ------------------------------------------------------------------ pooled outer products
@@ -342,24 +345,7 @@ int klhr_model_eval(const klhr_model_t* model, int dtype, const void* theta_dev,
     if (n_chains < 0) return fail(-10, "n_chains must be non-negative");
     if (n_chains == 0) return 0;
     if (!theta_dev || !lp_dev) return fail(-1, "theta and lp must not be NULL");
-    cudaStream_t st = (cudaStream_t)stream;
-    int e = -2;
-    switch (mp.id) {
-        case KLHR_MODEL_NORMAL: e = launch_eval_normal(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-        case KLHR_MODEL_ILL_NORMAL: e = launch_eval_ill_normal(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-        case KLHR_MODEL_FUNNEL: e = launch_eval_funnel(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-        case KLHR_MODEL_CORR_NORMAL: e = launch_eval_corr_normal(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-        case KLHR_MODEL_AR1: e = launch_eval_ar1(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-        case KLHR_MODEL_ARK: e = launch_eval_ark(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-        case KLHR_MODEL_ROSENBROCK: e = launch_eval_rosenbrock(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-        case KLHR_MODEL_EARNINGS: e = launch_eval_earnings(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-        case KLHR_MODEL_EIGHT_SCHOOLS_NC: e = launch_eval_eight_schools_nc(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-        case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_eval_eight_schools_c(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-        case KLHR_MODEL_LOGISTIC_REGRESSION: e = launch_eval_logistic_regression(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-        case KLHR_MODEL_ARMA11: e = launch_eval_arma11(mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-        case KLHR_MODEL_USER: e = user_table(mp).eval(&mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, st); break;
-    }
-    return cuda_fail(e, "klhr_model_eval");
+    return cuda_fail(launchers(mp).eval(&mp, dtype, theta_dev, lp_dev, grad_dev, n_chains, stream), "klhr_model_eval");
 }
 
 int klhr_step_replay(const klhr_model_t* model, const klhr_fit_t* fit, int dtype, void* theta_dev,
@@ -455,24 +441,7 @@ int klhr_mh_run(const klhr_model_t* model, int dtype, void* theta_dev, double st
     if (!theta_dev) return fail(-1, "theta must not be NULL");
     a.theta = theta_dev; a.B = n_chains; a.stepsize = stepsize;
     a.chain_offset = chain_offset; a.draw_offset = draw_offset; a.n_steps = n_steps; a.seed = seed;
-    cudaStream_t st = (cudaStream_t)stream;
-    int e = -2;
-    switch (a.mp.id) {
-        case KLHR_MODEL_NORMAL: e = launch_mh_normal(a, dtype, st); break;
-        case KLHR_MODEL_ILL_NORMAL: e = launch_mh_ill_normal(a, dtype, st); break;
-        case KLHR_MODEL_FUNNEL: e = launch_mh_funnel(a, dtype, st); break;
-        case KLHR_MODEL_CORR_NORMAL: e = launch_mh_corr_normal(a, dtype, st); break;
-        case KLHR_MODEL_AR1: e = launch_mh_ar1(a, dtype, st); break;
-        case KLHR_MODEL_ARK: e = launch_mh_ark(a, dtype, st); break;
-        case KLHR_MODEL_ROSENBROCK: e = launch_mh_rosenbrock(a, dtype, st); break;
-        case KLHR_MODEL_EARNINGS: e = launch_mh_earnings(a, dtype, st); break;
-        case KLHR_MODEL_EIGHT_SCHOOLS_NC: e = launch_mh_eight_schools_nc(a, dtype, st); break;
-        case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_mh_eight_schools_c(a, dtype, st); break;
-        case KLHR_MODEL_LOGISTIC_REGRESSION: e = launch_mh_logistic_regression(a, dtype, st); break;
-        case KLHR_MODEL_ARMA11: e = launch_mh_arma11(a, dtype, st); break;
-        case KLHR_MODEL_USER: e = user_table(a.mp).mh(&a, dtype, st); break;
-    }
-    return cuda_fail(e, "klhr_mh_run");
+    return cuda_fail(launchers(a.mp).mh(&a, dtype, stream), "klhr_mh_run");
 }
 
 static int check_slice(const klhr_slice_t* sp) {
@@ -482,25 +451,6 @@ static int check_slice(const klhr_slice_t* sp) {
     if (!(sp->tol >= 0)) return fail(-15, "slice: tol must be non-negative");
     if (sp->cap < 1) return fail(-15, "slice: cap must be >= 1");
     return 0;
-}
-
-static int dispatch_slice(const SliceArgs& a, int dtype, bool replay, cudaStream_t st) {
-    switch (a.mp.id) {
-        case KLHR_MODEL_NORMAL: return launch_slice_normal(a, dtype, replay, st);
-        case KLHR_MODEL_ILL_NORMAL: return launch_slice_ill_normal(a, dtype, replay, st);
-        case KLHR_MODEL_FUNNEL: return launch_slice_funnel(a, dtype, replay, st);
-        case KLHR_MODEL_CORR_NORMAL: return launch_slice_corr_normal(a, dtype, replay, st);
-        case KLHR_MODEL_AR1: return launch_slice_ar1(a, dtype, replay, st);
-        case KLHR_MODEL_ARK: return launch_slice_ark(a, dtype, replay, st);
-        case KLHR_MODEL_ROSENBROCK: return launch_slice_rosenbrock(a, dtype, replay, st);
-        case KLHR_MODEL_EARNINGS: return launch_slice_earnings(a, dtype, replay, st);
-        case KLHR_MODEL_EIGHT_SCHOOLS_NC: return launch_slice_eight_schools_nc(a, dtype, replay, st);
-        case KLHR_MODEL_EIGHT_SCHOOLS_C: return launch_slice_eight_schools_c(a, dtype, replay, st);
-        case KLHR_MODEL_LOGISTIC_REGRESSION: return launch_slice_logistic_regression(a, dtype, replay, st);
-        case KLHR_MODEL_ARMA11: return launch_slice_arma11(a, dtype, replay, st);
-        case KLHR_MODEL_USER: return user_table(a.mp).slice(&a, dtype, replay, st);
-    }
-    return -2;
 }
 
 int klhr_slice_run(const klhr_model_t* model, const klhr_slice_t* slice, const klhr_direction_t* dir, int dtype,
@@ -533,7 +483,7 @@ int klhr_slice_run(const klhr_model_t* model, const klhr_slice_t* slice, const k
     a.sp = *slice; a.tol = slice->tol;
     a.theta = theta_dev; a.B = n_chains;
     a.chain_offset = chain_offset; a.draw_offset = draw_offset; a.n_steps = n_steps; a.seed = seed;
-    return cuda_fail(dispatch_slice(a, dtype, false, (cudaStream_t)stream), "klhr_slice_run");
+    return cuda_fail(launchers(a.mp).slice(&a, dtype, false, stream), "klhr_slice_run");
 }
 
 int klhr_slice_replay(const klhr_model_t* model, const klhr_slice_t* slice, int dtype, void* theta_dev,
@@ -555,7 +505,7 @@ int klhr_slice_replay(const klhr_model_t* model, const klhr_slice_t* slice, int 
     a.acc.thin = 1;
     if (trace) a.tr = *trace;
     a.tr.slice_u = nullptr;                                       // input in this mode
-    return cuda_fail(dispatch_slice(a, dtype, true, (cudaStream_t)stream), "klhr_slice_replay");
+    return cuda_fail(launchers(a.mp).slice(&a, dtype, true, stream), "klhr_slice_replay");
 }
 
 int klhr_kl_eval(const klhr_model_t* model, const klhr_fit_t* fit, int dtype, const void* theta_dev,
@@ -572,24 +522,7 @@ int klhr_kl_eval(const klhr_model_t* model, const klhr_fit_t* fit, int dtype, co
         return fail(-1, "theta, rho, eta, f, grad must not be NULL");
     a.theta = theta_dev; a.rho = rho_dev; a.eta = eta_dev; a.f = f_dev; a.grad = grad_dev; a.hess = hess_dev;
     a.B = n_chains;
-    cudaStream_t st = (cudaStream_t)stream;
-    int e = -2;
-    switch (a.mp.id) {
-        case KLHR_MODEL_NORMAL: e = launch_kl_normal(a, dtype, fit->family, st); break;
-        case KLHR_MODEL_ILL_NORMAL: e = launch_kl_ill_normal(a, dtype, fit->family, st); break;
-        case KLHR_MODEL_FUNNEL: e = launch_kl_funnel(a, dtype, fit->family, st); break;
-        case KLHR_MODEL_CORR_NORMAL: e = launch_kl_corr_normal(a, dtype, fit->family, st); break;
-        case KLHR_MODEL_AR1: e = launch_kl_ar1(a, dtype, fit->family, st); break;
-        case KLHR_MODEL_ARK: e = launch_kl_ark(a, dtype, fit->family, st); break;
-        case KLHR_MODEL_ROSENBROCK: e = launch_kl_rosenbrock(a, dtype, fit->family, st); break;
-        case KLHR_MODEL_EARNINGS: e = launch_kl_earnings(a, dtype, fit->family, st); break;
-        case KLHR_MODEL_EIGHT_SCHOOLS_NC: e = launch_kl_eight_schools_nc(a, dtype, fit->family, st); break;
-        case KLHR_MODEL_EIGHT_SCHOOLS_C: e = launch_kl_eight_schools_c(a, dtype, fit->family, st); break;
-        case KLHR_MODEL_LOGISTIC_REGRESSION: e = launch_kl_logistic_regression(a, dtype, fit->family, st); break;
-        case KLHR_MODEL_ARMA11: e = launch_kl_arma11(a, dtype, fit->family, st); break;
-        case KLHR_MODEL_USER: e = user_table(a.mp).kl(&a, dtype, fit->family, st); break;
-    }
-    return cuda_fail(e, "klhr_kl_eval");
+    return cuda_fail(launchers(a.mp).kl(&a, dtype, fit->family, stream), "klhr_kl_eval");
 }
 
 // ---- elementwise fp64 exp / log of the fit's inner loops (klhr_math.cuh), exposed for the accuracy tests

@@ -363,27 +363,4 @@ int launch_chain_typed(const StepArgs& args_in, int family, bool replay, cudaStr
     return (int)e;
 }
 
-#define KLHR_DECLARE_MODEL_CHAIN(name) \
-    int launch_chain_##name(const StepArgs& a, int dtype, int family, bool replay, cudaStream_t st, LaunchInfo* info);
-
-#define KLHR_DEFINE_MODEL_CHAIN(name, M64, M32)                                                              \
-    int launch_chain_##name(const StepArgs& a, int dtype, int family, bool replay, cudaStream_t st,          \
-                            LaunchInfo* info) {                                                              \
-        return dtype == KLHR_F64 ? launch_chain_typed<double, M64>(a, family, replay, st, info)              \
-                                 : launch_chain_typed<float, M32>(a, family, replay, st, info);              \
-    }
-
-KLHR_DECLARE_MODEL_CHAIN(normal)
-KLHR_DECLARE_MODEL_CHAIN(ill_normal)
-KLHR_DECLARE_MODEL_CHAIN(funnel)
-KLHR_DECLARE_MODEL_CHAIN(corr_normal)
-KLHR_DECLARE_MODEL_CHAIN(ar1)
-KLHR_DECLARE_MODEL_CHAIN(ark)
-KLHR_DECLARE_MODEL_CHAIN(rosenbrock)
-KLHR_DECLARE_MODEL_CHAIN(earnings)
-KLHR_DECLARE_MODEL_CHAIN(eight_schools_nc)
-KLHR_DECLARE_MODEL_CHAIN(eight_schools_c)
-KLHR_DECLARE_MODEL_CHAIN(logistic_regression)
-KLHR_DECLARE_MODEL_CHAIN(arma11)
-
 }  // namespace klhr

@@ -130,23 +130,4 @@ int launch_mh_typed(const MhArgs& args_in, cudaStream_t st) {
     return (int)cudaLaunchKernel(fn, dim3((unsigned)grid), dim3((unsigned)threads), kargs, smem, st);
 }
 
-#define KLHR_DECLARE_MODEL_MH(name) int launch_mh_##name(const MhArgs& a, int dtype, cudaStream_t st);
-#define KLHR_DEFINE_MODEL_MH(name, M64, M32)                                             \
-    int launch_mh_##name(const MhArgs& a, int dtype, cudaStream_t st) {                  \
-        return dtype == KLHR_F64 ? launch_mh_typed<double, M64>(a, st) : launch_mh_typed<float, M32>(a, st); \
-    }
-
-KLHR_DECLARE_MODEL_MH(normal)
-KLHR_DECLARE_MODEL_MH(ill_normal)
-KLHR_DECLARE_MODEL_MH(funnel)
-KLHR_DECLARE_MODEL_MH(corr_normal)
-KLHR_DECLARE_MODEL_MH(ar1)
-KLHR_DECLARE_MODEL_MH(ark)
-KLHR_DECLARE_MODEL_MH(rosenbrock)
-KLHR_DECLARE_MODEL_MH(earnings)
-KLHR_DECLARE_MODEL_MH(eight_schools_nc)
-KLHR_DECLARE_MODEL_MH(eight_schools_c)
-KLHR_DECLARE_MODEL_MH(logistic_regression)
-KLHR_DECLARE_MODEL_MH(arma11)
-
 }  // namespace klhr

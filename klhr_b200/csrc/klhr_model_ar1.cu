@@ -1,14 +1,7 @@
-// klhr_b200 -- step/eval kernel instantiations for one Stan target (one translation unit
+// klhr_b200 -- the launcher table of one Stan target, which instantiates every kernel for it (one translation unit
 // per model so the build parallelises).  See klhr_models.cuh for the density itself.
-#include "klhr_chain.cuh"
-#include "klhr_mh.cuh"
-#include "klhr_slice.cuh"
+#include "klhr_target.cuh"
 
 namespace klhr {
-using M64_ar1 = AR1<double>;
-using M32_ar1 = AR1<float>;
-KLHR_DEFINE_MODEL(ar1, M64_ar1, M32_ar1)
-KLHR_DEFINE_MODEL_CHAIN(ar1, M64_ar1, M32_ar1)
-KLHR_DEFINE_MODEL_MH(ar1, M64_ar1, M32_ar1)
-KLHR_DEFINE_MODEL_SLICE(ar1, M64_ar1, M32_ar1)
+extern const klhr_user_table_t kAr1Launchers = TargetLaunchers<AR1<double>, AR1<float>>::table;
 }  // namespace klhr

@@ -1,14 +1,7 @@
-// klhr_b200 -- step/eval kernel instantiations for one Stan target (one translation unit
+// klhr_b200 -- the launcher table of one Stan target, which instantiates every kernel for it (one translation unit
 // per model so the build parallelises).  See klhr_models.cuh for the density itself.
-#include "klhr_chain.cuh"
-#include "klhr_mh.cuh"
-#include "klhr_slice.cuh"
+#include "klhr_target.cuh"
 
 namespace klhr {
-using M64_ark = ARK<double>;
-using M32_ark = ARK<float>;
-KLHR_DEFINE_MODEL(ark, M64_ark, M32_ark)
-KLHR_DEFINE_MODEL_CHAIN(ark, M64_ark, M32_ark)
-KLHR_DEFINE_MODEL_MH(ark, M64_ark, M32_ark)
-KLHR_DEFINE_MODEL_SLICE(ark, M64_ark, M32_ark)
+extern const klhr_user_table_t kArkLaunchers = TargetLaunchers<ARK<double>, ARK<float>>::table;
 }  // namespace klhr

@@ -1,14 +1,7 @@
-// klhr_b200 -- step/eval kernel instantiations for one Stan target (one translation unit
+// klhr_b200 -- the launcher table of one Stan target, which instantiates every kernel for it (one translation unit
 // per model so the build parallelises).  See klhr_models.cuh for the density itself.
-#include "klhr_chain.cuh"
-#include "klhr_mh.cuh"
-#include "klhr_slice.cuh"
+#include "klhr_target.cuh"
 
 namespace klhr {
-using M64_arma11 = Arma11<double>;
-using M32_arma11 = Arma11<float>;
-KLHR_DEFINE_MODEL(arma11, M64_arma11, M32_arma11)
-KLHR_DEFINE_MODEL_CHAIN(arma11, M64_arma11, M32_arma11)
-KLHR_DEFINE_MODEL_MH(arma11, M64_arma11, M32_arma11)
-KLHR_DEFINE_MODEL_SLICE(arma11, M64_arma11, M32_arma11)
+extern const klhr_user_table_t kArma11Launchers = TargetLaunchers<Arma11<double>, Arma11<float>>::table;
 }  // namespace klhr

@@ -1,14 +1,7 @@
-// klhr_b200 -- step/eval kernel instantiations for one Stan target (one translation unit
+// klhr_b200 -- the launcher table of one Stan target, which instantiates every kernel for it (one translation unit
 // per model so the build parallelises).  See klhr_models.cuh for the density itself.
-#include "klhr_chain.cuh"
-#include "klhr_mh.cuh"
-#include "klhr_slice.cuh"
+#include "klhr_target.cuh"
 
 namespace klhr {
-using M64_corr_normal = CorrNormal<double>;
-using M32_corr_normal = CorrNormal<float>;
-KLHR_DEFINE_MODEL(corr_normal, M64_corr_normal, M32_corr_normal)
-KLHR_DEFINE_MODEL_CHAIN(corr_normal, M64_corr_normal, M32_corr_normal)
-KLHR_DEFINE_MODEL_MH(corr_normal, M64_corr_normal, M32_corr_normal)
-KLHR_DEFINE_MODEL_SLICE(corr_normal, M64_corr_normal, M32_corr_normal)
+extern const klhr_user_table_t kCorrNormalLaunchers = TargetLaunchers<CorrNormal<double>, CorrNormal<float>>::table;
 }  // namespace klhr

@@ -1,14 +1,7 @@
-// klhr_b200 -- step/eval kernel instantiations for one Stan target (one translation unit
+// klhr_b200 -- the launcher table of one Stan target, which instantiates every kernel for it (one translation unit
 // per model so the build parallelises).  See klhr_models.cuh for the density itself.
-#include "klhr_chain.cuh"
-#include "klhr_mh.cuh"
-#include "klhr_slice.cuh"
+#include "klhr_target.cuh"
 
 namespace klhr {
-using M64_earnings = Earnings<double>;
-using M32_earnings = Earnings<float>;
-KLHR_DEFINE_MODEL(earnings, M64_earnings, M32_earnings)
-KLHR_DEFINE_MODEL_CHAIN(earnings, M64_earnings, M32_earnings)
-KLHR_DEFINE_MODEL_MH(earnings, M64_earnings, M32_earnings)
-KLHR_DEFINE_MODEL_SLICE(earnings, M64_earnings, M32_earnings)
+extern const klhr_user_table_t kEarningsLaunchers = TargetLaunchers<Earnings<double>, Earnings<float>>::table;
 }  // namespace klhr

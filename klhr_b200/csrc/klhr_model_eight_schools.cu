@@ -1,22 +1,11 @@
-// klhr_b200 -- step/eval kernel instantiations for one Stan target (one translation unit
+// klhr_b200 -- the launcher table of one Stan target, which instantiates every kernel for it (one translation unit
 // per model so the build parallelises).  See klhr_models.cuh for the density itself.
 // Both parametrisations of eight schools share this unit: they are small and read the same data.
-#include "klhr_chain.cuh"
-#include "klhr_mh.cuh"
-#include "klhr_slice.cuh"
+#include "klhr_target.cuh"
 
 namespace klhr {
-using M64_eight_schools_nc = EightSchoolsNC<double>;
-using M32_eight_schools_nc = EightSchoolsNC<float>;
-KLHR_DEFINE_MODEL(eight_schools_nc, M64_eight_schools_nc, M32_eight_schools_nc)
-KLHR_DEFINE_MODEL_CHAIN(eight_schools_nc, M64_eight_schools_nc, M32_eight_schools_nc)
-KLHR_DEFINE_MODEL_MH(eight_schools_nc, M64_eight_schools_nc, M32_eight_schools_nc)
-KLHR_DEFINE_MODEL_SLICE(eight_schools_nc, M64_eight_schools_nc, M32_eight_schools_nc)
-
-using M64_eight_schools_c = EightSchoolsC<double>;
-using M32_eight_schools_c = EightSchoolsC<float>;
-KLHR_DEFINE_MODEL(eight_schools_c, M64_eight_schools_c, M32_eight_schools_c)
-KLHR_DEFINE_MODEL_CHAIN(eight_schools_c, M64_eight_schools_c, M32_eight_schools_c)
-KLHR_DEFINE_MODEL_MH(eight_schools_c, M64_eight_schools_c, M32_eight_schools_c)
-KLHR_DEFINE_MODEL_SLICE(eight_schools_c, M64_eight_schools_c, M32_eight_schools_c)
+extern const klhr_user_table_t kEightSchoolsNCLaunchers =
+    TargetLaunchers<EightSchoolsNC<double>, EightSchoolsNC<float>>::table;
+extern const klhr_user_table_t kEightSchoolsCLaunchers =
+    TargetLaunchers<EightSchoolsC<double>, EightSchoolsC<float>>::table;
 }  // namespace klhr

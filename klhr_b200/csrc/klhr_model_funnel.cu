@@ -1,14 +1,7 @@
-// klhr_b200 -- step/eval kernel instantiations for one Stan target (one translation unit
+// klhr_b200 -- the launcher table of one Stan target, which instantiates every kernel for it (one translation unit
 // per model so the build parallelises).  See klhr_models.cuh for the density itself.
-#include "klhr_chain.cuh"
-#include "klhr_mh.cuh"
-#include "klhr_slice.cuh"
+#include "klhr_target.cuh"
 
 namespace klhr {
-using M64_funnel = Funnel<double>;
-using M32_funnel = Funnel<float>;
-KLHR_DEFINE_MODEL(funnel, M64_funnel, M32_funnel)
-KLHR_DEFINE_MODEL_CHAIN(funnel, M64_funnel, M32_funnel)
-KLHR_DEFINE_MODEL_MH(funnel, M64_funnel, M32_funnel)
-KLHR_DEFINE_MODEL_SLICE(funnel, M64_funnel, M32_funnel)
+extern const klhr_user_table_t kFunnelLaunchers = TargetLaunchers<Funnel<double>, Funnel<float>>::table;
 }  // namespace klhr

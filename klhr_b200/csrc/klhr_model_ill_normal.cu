@@ -1,14 +1,8 @@
-// klhr_b200 -- step/eval kernel instantiations for one Stan target (one translation unit
+// klhr_b200 -- the launcher table of one Stan target, which instantiates every kernel for it (one translation unit
 // per model so the build parallelises).  See klhr_models.cuh for the density itself.
-#include "klhr_chain.cuh"
-#include "klhr_mh.cuh"
-#include "klhr_slice.cuh"
+#include "klhr_target.cuh"
 
 namespace klhr {
-using M64_ill_normal = DiagNormal<double,true>;
-using M32_ill_normal = DiagNormal<float,true>;
-KLHR_DEFINE_MODEL(ill_normal, M64_ill_normal, M32_ill_normal)
-KLHR_DEFINE_MODEL_CHAIN(ill_normal, M64_ill_normal, M32_ill_normal)
-KLHR_DEFINE_MODEL_MH(ill_normal, M64_ill_normal, M32_ill_normal)
-KLHR_DEFINE_MODEL_SLICE(ill_normal, M64_ill_normal, M32_ill_normal)
+extern const klhr_user_table_t kIllNormalLaunchers =
+    TargetLaunchers<DiagNormal<double, true>, DiagNormal<float, true>>::table;
 }  // namespace klhr

@@ -1,14 +1,8 @@
-// klhr_b200 -- step/eval kernel instantiations for one Stan target (one translation unit
+// klhr_b200 -- the launcher table of one Stan target, which instantiates every kernel for it (one translation unit
 // per model so the build parallelises).  See klhr_models.cuh for the density itself.
-#include "klhr_chain.cuh"
-#include "klhr_mh.cuh"
-#include "klhr_slice.cuh"
+#include "klhr_target.cuh"
 
 namespace klhr {
-using M64_normal = DiagNormal<double,false>;
-using M32_normal = DiagNormal<float,false>;
-KLHR_DEFINE_MODEL(normal, M64_normal, M32_normal)
-KLHR_DEFINE_MODEL_CHAIN(normal, M64_normal, M32_normal)
-KLHR_DEFINE_MODEL_MH(normal, M64_normal, M32_normal)
-KLHR_DEFINE_MODEL_SLICE(normal, M64_normal, M32_normal)
+extern const klhr_user_table_t kNormalLaunchers =
+    TargetLaunchers<DiagNormal<double, false>, DiagNormal<float, false>>::table;
 }  // namespace klhr

@@ -1,14 +1,7 @@
-// klhr_b200 -- step/eval kernel instantiations for one Stan target (one translation unit
+// klhr_b200 -- the launcher table of one Stan target, which instantiates every kernel for it (one translation unit
 // per model so the build parallelises).  See klhr_models.cuh for the density itself.
-#include "klhr_chain.cuh"
-#include "klhr_mh.cuh"
-#include "klhr_slice.cuh"
+#include "klhr_target.cuh"
 
 namespace klhr {
-using M64_rosenbrock = Rosenbrock<double>;
-using M32_rosenbrock = Rosenbrock<float>;
-KLHR_DEFINE_MODEL(rosenbrock, M64_rosenbrock, M32_rosenbrock)
-KLHR_DEFINE_MODEL_CHAIN(rosenbrock, M64_rosenbrock, M32_rosenbrock)
-KLHR_DEFINE_MODEL_MH(rosenbrock, M64_rosenbrock, M32_rosenbrock)
-KLHR_DEFINE_MODEL_SLICE(rosenbrock, M64_rosenbrock, M32_rosenbrock)
+extern const klhr_user_table_t kRosenbrockLaunchers = TargetLaunchers<Rosenbrock<double>, Rosenbrock<float>>::table;
 }  // namespace klhr

@@ -218,24 +218,4 @@ int launch_slice_typed(const SliceArgs& args_in, bool replay, cudaStream_t st) {
     return (int)cudaLaunchKernel(fn, dim3((unsigned)grid), dim3((unsigned)threads), kargs, smem, st);
 }
 
-#define KLHR_DECLARE_MODEL_SLICE(name) int launch_slice_##name(const SliceArgs& a, int dtype, bool replay, cudaStream_t st);
-#define KLHR_DEFINE_MODEL_SLICE(name, M64, M32)                                                    \
-    int launch_slice_##name(const SliceArgs& a, int dtype, bool replay, cudaStream_t st) {         \
-        return dtype == KLHR_F64 ? launch_slice_typed<double, M64>(a, replay, st)                  \
-                                 : launch_slice_typed<float, M32>(a, replay, st);                  \
-    }
-
-KLHR_DECLARE_MODEL_SLICE(normal)
-KLHR_DECLARE_MODEL_SLICE(ill_normal)
-KLHR_DECLARE_MODEL_SLICE(funnel)
-KLHR_DECLARE_MODEL_SLICE(corr_normal)
-KLHR_DECLARE_MODEL_SLICE(ar1)
-KLHR_DECLARE_MODEL_SLICE(ark)
-KLHR_DECLARE_MODEL_SLICE(rosenbrock)
-KLHR_DECLARE_MODEL_SLICE(earnings)
-KLHR_DECLARE_MODEL_SLICE(eight_schools_nc)
-KLHR_DECLARE_MODEL_SLICE(eight_schools_c)
-KLHR_DECLARE_MODEL_SLICE(logistic_regression)
-KLHR_DECLARE_MODEL_SLICE(arma11)
-
 }  // namespace klhr

@@ -551,41 +551,4 @@ int launch_eval_typed(const ModelParams& mp, const void* theta, void* lp, void* 
     return (int)cudaGetLastError();
 }
 
-// per-model launchers, one translation unit each (klhr_model_*.cu)
-#define KLHR_DECLARE_MODEL(name)                                                                      \
-    int launch_step_##name(const StepArgs& a, int dtype, int family, bool replay, bool accum,         \
-                           cudaStream_t st, LaunchInfo* info);                                        \
-    int launch_eval_##name(const ModelParams& mp, int dtype, const void* theta, void* lp, void* grad, \
-                           long long B, cudaStream_t st);                                             \
-    int launch_kl_##name(const KlArgs& a, int dtype, int family, cudaStream_t st);
-
-#define KLHR_DEFINE_MODEL(name, M64, M32)                                                             \
-    int launch_step_##name(const StepArgs& a, int dtype, int family, bool replay, bool accum,         \
-                           cudaStream_t st, LaunchInfo* info) {                                       \
-        return dtype == KLHR_F64 ? launch_step_typed<double, M64>(a, family, replay, accum, st, info) \
-                                 : launch_step_typed<float, M32>(a, family, replay, accum, st, info); \
-    }                                                                                                 \
-    int launch_eval_##name(const ModelParams& mp, int dtype, const void* theta, void* lp, void* grad, \
-                           long long B, cudaStream_t st) {                                            \
-        return dtype == KLHR_F64 ? launch_eval_typed<double, M64>(mp, theta, lp, grad, B, st)         \
-                                 : launch_eval_typed<float, M32>(mp, theta, lp, grad, B, st);         \
-    }                                                                                                 \
-    int launch_kl_##name(const KlArgs& a, int dtype, int family, cudaStream_t st) {                   \
-        return dtype == KLHR_F64 ? launch_kl_typed<double, M64>(a, family, st)                        \
-                                 : launch_kl_typed<float, M32>(a, family, st);                        \
-    }
-
-KLHR_DECLARE_MODEL(normal)
-KLHR_DECLARE_MODEL(ill_normal)
-KLHR_DECLARE_MODEL(funnel)
-KLHR_DECLARE_MODEL(corr_normal)
-KLHR_DECLARE_MODEL(ar1)
-KLHR_DECLARE_MODEL(ark)
-KLHR_DECLARE_MODEL(rosenbrock)
-KLHR_DECLARE_MODEL(earnings)
-KLHR_DECLARE_MODEL(eight_schools_nc)
-KLHR_DECLARE_MODEL(eight_schools_c)
-KLHR_DECLARE_MODEL(logistic_regression)
-KLHR_DECLARE_MODEL(arma11)
-
 }  // namespace klhr

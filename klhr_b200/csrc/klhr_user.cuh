@@ -27,9 +27,7 @@
 // passes and one plain pass on every evaluation where it is active.
 #pragma once
 #include "klhr_ad.cuh"
-#include "klhr_chain.cuh"
-#include "klhr_mh.cuh"
-#include "klhr_slice.cuh"
+#include "klhr_target.cuh"
 #include "../../include/klhr_user.h"
 
 namespace klhr {
@@ -112,40 +110,7 @@ struct UserModel {
 
 // Instantiates every kernel for UserModel<double, Target> and UserModel<float, Target> and exports the launcher table
 // (include/klhr_user.h).  The generated translation unit of a user target ends with this macro.
-#define KLHR_DEFINE_USER_TARGET(TARGET)                                                                               \
-    namespace klhr {                                                                                                  \
-    using UserM64 = UserModel<double, TARGET>;                                                                        \
-    using UserM32 = UserModel<float, TARGET>;                                                                         \
-    KLHR_DEFINE_MODEL(user, UserM64, UserM32)                                                                         \
-    KLHR_DEFINE_MODEL_CHAIN(user, UserM64, UserM32)                                                                   \
-    KLHR_DEFINE_MODEL_MH(user, UserM64, UserM32)                                                                      \
-    KLHR_DEFINE_MODEL_SLICE(user, UserM64, UserM32)                                                                   \
-    static int user_step(const void* a, int dtype, int family, int replay, int accum, void* st, void* info) {         \
-        return launch_step_user(*static_cast<const StepArgs*>(a), dtype, family, replay != 0, accum != 0,             \
-                                static_cast<cudaStream_t>(st), static_cast<LaunchInfo*>(info));                       \
-    }                                                                                                                 \
-    static int user_chain(const void* a, int dtype, int family, int replay, void* st, void* info) {                   \
-        return launch_chain_user(*static_cast<const StepArgs*>(a), dtype, family, replay != 0,                        \
-                                 static_cast<cudaStream_t>(st), static_cast<LaunchInfo*>(info));                      \
-    }                                                                                                                 \
-    static int user_eval(const void* mp, int dtype, const void* theta, void* lp, void* grad, int64_t B, void* st) {   \
-        return launch_eval_user(*static_cast<const ModelParams*>(mp), dtype, theta, lp, grad, B,                      \
-                                static_cast<cudaStream_t>(st));                                                       \
-    }                                                                                                                 \
-    static int user_kl(const void* a, int dtype, int family, void* st) {                                              \
-        return launch_kl_user(*static_cast<const KlArgs*>(a), dtype, family, static_cast<cudaStream_t>(st));          \
-    }                                                                                                                 \
-    static int user_mh(const void* a, int dtype, void* st) {                                                          \
-        return launch_mh_user(*static_cast<const MhArgs*>(a), dtype, static_cast<cudaStream_t>(st));                  \
-    }                                                                                                                 \
-    static int user_slice(const void* a, int dtype, int replay, void* st) {                                           \
-        return launch_slice_user(*static_cast<const SliceArgs*>(a), dtype, replay != 0, static_cast<cudaStream_t>(st)); \
-    }                                                                                                                 \
-    static const klhr_user_table_t kUserTable = {                                                                     \
-        KLHR_ABI_VERSION, (int32_t)sizeof(StepArgs), (int32_t)sizeof(SliceArgs), (int32_t)sizeof(MhArgs),             \
-        (int32_t)sizeof(KlArgs), (int32_t)sizeof(ModelParams),                                                        \
-        user_step, user_chain, user_eval, user_kl, user_mh, user_slice};                                              \
-    }                                                                                                                 \
-    extern "C" __attribute__((visibility("default"))) const klhr_user_table_t* klhr_user_table(void) {                \
-        return &klhr::kUserTable;                                                                                     \
+#define KLHR_DEFINE_USER_TARGET(TARGET)                                                                        \
+    extern "C" __attribute__((visibility("default"))) const klhr_user_table_t* klhr_user_table(void) {         \
+        return &klhr::TargetLaunchers<klhr::UserModel<double, TARGET>, klhr::UserModel<float, TARGET>>::table; \
     }
